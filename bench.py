@@ -1,6 +1,6 @@
 """bench.py — headline benchmark of the aggregation path (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload rmat26]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload rmat26] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[4], the configuration the metric's "at 1/2/4/8 B200"
 is quoted on: dst-partitioned gather->scatter_add on a synthetic R-MAT scale-26 graph
@@ -18,7 +18,8 @@ CUDA-event time against MEASURED_PEAKS.json; `parity` = this run's output checke
 fp64 index_add_ of the same inputs on every rank; `per_config` (N=1) = kernel fractions of the
 other BASELINE.json configs (C1, products, Reddit-shaped fp32/bf16, C4) from the same run.
 `--workload products` keeps round 1's configs[1] bench (weak scaling at N>1).
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  `--dump-outputs DIR` also writes the output of the last timed
+step (a fixed, seeded sample of its rows) as .npy files; nothing else is written.
 """
 import argparse
 import json
@@ -34,6 +35,7 @@ for _p in (ROOT, os.path.join(ROOT, "gnn-ops-benchmark_b200")):
     if _p not in sys.path:
         sys.path.insert(0, _p)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 WORKLOADS = {
@@ -397,6 +399,28 @@ def parity_check(out, x_of, src, dst, row0, n_rows, tol, block_rows=1 << 21, edg
     return worst
 
 
+# ---------------------------------------------------------------------- --dump-outputs --
+DUMP_BYTES = 32 << 20   # all ranks together; well under 64 MB with the row ids and .npy headers
+
+
+def dump_outputs(dirname, out, row0, rank, world):
+    """Writes this rank's output rows of the last timed step as float32 to DIR/out.npy, with
+    their global row ids as float64 to DIR/out_rows.npy (suffix _rank<r> at N > 1).  Outputs
+    larger than the budget are represented by a fixed, seeded sample of rows, so two builds run
+    with the same arguments can be compared output for output."""
+    n_rows, F = out.shape
+    k = min(n_rows, DUMP_BYTES // world // (F * 4 + 8))
+    if k == n_rows:
+        rows = torch.arange(n_rows)
+    else:
+        rows = torch.randperm(n_rows, generator=torch.Generator().manual_seed(20240601))[:k].sort().values
+    vals = out.index_select(0, rows.to(out.device)).float().cpu().numpy()
+    suffix = "" if world == 1 else f"_rank{rank}"
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, f"out{suffix}.npy"), vals)
+    np.save(os.path.join(dirname, f"out_rows{suffix}.npy"), (rows + row0).double().numpy())
+
+
 # ------------------------------------------------------------------------ per_config --
 def per_config(iters):
     """Kernel times / roofline fractions of the other BASELINE.json configs (profiles/bench_ops.py
@@ -558,6 +582,8 @@ def run_rmat(args):
     sampler.mark()
     launches = gno_b200.launch_count() - launches0
     total_ms = a.elapsed_time(b)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, lo, rank, world)
 
     # ---- kernel-only: this rank's segment-reduce launches, no exchange (the roofline kernel) ----
     x_gather = x_local if world == 1 else (recv if recv is not None else agg._push_buffer(F, dtype, dev)[0][:n_needed])
@@ -849,6 +875,8 @@ def run_weak(args):
     sampler.mark()
     launches = gno_b200.launch_count() - launches0
     total_ms = ev[0].elapsed_time(ev[1])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, rank * n_local, rank, world)
     if world > 1:
         t = torch.tensor([total_ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -1047,7 +1075,12 @@ def main():
                     help="grid cap of the push kernel when it runs beside the reduction (0 = fill the chip)")
     ap.add_argument("--per-config", type=int, default=1,
                     help="N=1: also time the other BASELINE.json configs' kernels (per_config object)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the output of the last timed step to DIR/*.npy (float32, a fixed seeded "
+                         "sample of rows when larger than 32 MB) for output-for-output comparison of builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     elif is_rmat(args.workload):

@@ -61,6 +61,36 @@ def test_rmat_slice_sampler_matches_the_full_graph():
         assert abs(got - want) < 0.01
 
 
+def test_dump_outputs_sample_and_budget(tmp_path):
+    """--dump-outputs: float32 rows with float64 global row ids, every row of a small output, the
+    same seeded sample of a large one on every call, and the whole dump under 64 MB."""
+    import numpy as np
+    import bench as B
+    small = torch.randn(100, 8, dtype=torch.bfloat16)
+    B.dump_outputs(str(tmp_path / "s"), small, 0, 0, 1)
+    v, r = np.load(tmp_path / "s" / "out.npy"), np.load(tmp_path / "s" / "out_rows.npy")
+    assert v.dtype == np.float32 and r.dtype == np.float64
+    assert np.array_equal(v, small.float().numpy()) and np.array_equal(r, np.arange(100.0))
+    big = torch.arange(300_000, dtype=torch.float32)[:, None].expand(-1, 64).contiguous()
+    for d in ("a", "b"):
+        for rank in range(2):
+            B.dump_outputs(str(tmp_path / d), big, 1000 + rank, rank, 2)
+    for rank in range(2):
+        va, ra = (np.load(tmp_path / "a" / f"{n}_rank{rank}.npy") for n in ("out", "out_rows"))
+        vb, rb = (np.load(tmp_path / "b" / f"{n}_rank{rank}.npy") for n in ("out", "out_rows"))
+        assert np.array_equal(va, vb) and np.array_equal(ra, rb)
+        assert 0 < len(ra) < 300_000 and np.all(np.diff(ra) > 0)
+        assert np.array_equal(va[:, 0], ra - 1000 - rank)         # each row is the output row its id names
+    total = sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir())
+    assert total <= 64 << 20
+
+
+def test_steps_must_be_positive():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload",
+                        "rmat16", "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr and r.stdout.strip() == ""
+
+
 def test_parity_check_detects_errors():
     import bench as B
     g = torch.Generator().manual_seed(0)
