@@ -39,6 +39,11 @@ constexpr int kSegWarps = kSegThreads / 32;
 #define GNO_SEG_INFLIGHT 64  // bytes of gathered rows in flight per lane (sets the unroll U)
 #endif
 constexpr int kSegMinBlocks = GNO_SEG_MINB;
+// per-head weights are one more gathered value per edge and lane: 80 registers (24 warps/SM) keep
+// the unrolled batch of gathers and weights out of local memory; the shuffle-staged kernel with
+// 16-bit data in 16-byte vectors needs 96 (20 warps/SM)
+constexpr int kSegMinBlocksHeads = 6;
+constexpr int kSegMinBlocksHeadsWide = 5;
 constexpr int kNoArg = INT_MAX;
 
 struct SegParams {
@@ -70,6 +75,8 @@ struct SegParams {
   int tma_ok;     // edge-record arrays are 16-byte aligned (bulk copies allowed)
   int staged;     // use the TMA-staged kernel (record slab of a CTA fits the shared-memory budget)
   unsigned x2_first;  // 0xffffffff when there is no second base (no gather id reaches it)
+  int H;              // per-head weights (gno_segment_reduce_heads): w is [*, H], read at w[eid * H + h]
+  int head_c;         // columns per head; a gathered vector never straddles two heads
 };
 
 // Address of row `idx` of the gather source: two bases, one compare and a select (xcol2 is
@@ -369,8 +376,12 @@ __device__ __forceinline__ void flush_acc(const SegParams& p, int row, int chunk
   }
 }
 
-template <typename T, int VB, int RED, bool ARG, bool HAS_W, int U>
-__global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMinBlocks - 1 : kSegMinBlocks)
+// HEADS (with HAS_W): the weight of a lane's vector is w[eid[k] * H + h] for the head h its columns
+// belong to, gathered per lane through the original edge id instead of staged per sorted edge.
+template <typename T, int VB, int RED, bool ARG, bool HAS_W, int U, bool HEADS = false>
+__global__ void __launch_bounds__(kSegThreads,
+                                  HEADS ? (sizeof(T) == 2 && VB == 16 ? kSegMinBlocksHeadsWide : kSegMinBlocksHeads)
+                                        : (ARG || sizeof(T) == 2) ? kSegMinBlocks - 1 : kSegMinBlocks)
     segreduce_kernel(const SegParams p) {
   // programmatic dependent launch: the finish kernel may become resident while the last wave runs
   // (it fills the empty rows, then waits for this grid before touching the chunk partials)
@@ -400,7 +411,8 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
   const int32_t* erow = p.erow + k0;
   const int32_t* gidx = p.gidx ? p.gidx + k0 : nullptr;
   const int32_t* eid = p.eid ? p.eid + k0 : nullptr;
-  const T* wgt = HAS_W ? static_cast<const T*>(p.w) + k0 : nullptr;
+  const T* wgt = (HAS_W && !HEADS) ? static_cast<const T*>(p.w) + k0 : nullptr;
+  const T* whead = HEADS ? static_cast<const T*>(p.w) + (v * EPV) / p.head_c : nullptr;
 
   Accum<T, VB, RED, HAS_W> acc;
   int ae[ARG ? EPV : 1];
@@ -421,12 +433,12 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
       s_row = stream_idx ? ld_stream_i32(erow + k, pol_stream) : __ldg(erow + k);
       if (gidx) s_idx = stream_idx ? ld_stream_i32(gidx + k, pol_stream) : __ldg(gidx + k);
       else s_idx = (int)(k0 + k);
-      if constexpr (ARG) {
+      if constexpr (ARG || HEADS) {
         if (p.eid == p.gidx) s_e = s_idx;
         else if (eid) s_e = stream_idx ? ld_stream_i32(eid + k, pol_stream) : __ldg(eid + k);
         else s_e = (int)(k0 + k);
       }
-      if constexpr (HAS_W) s_w = DType<T>::to_f(wgt[k]);
+      if constexpr (HAS_W && !HEADS) s_w = DType<T>::to_f(wgt[k]);
     }
   };
 
@@ -446,14 +458,15 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
     if (ti + 1 < ntiles) stage(t + G, nx_idx, nx_row, nx_e, nx_w);
     for (int j = 0; j < G; j += U) {
       Words<VB> val[U];
-      int e_u[ARG ? U : 1];
+      int e_u[(ARG || HEADS) ? U : 1];
       float w_u[HAS_W ? U : 1];
       const int lane0 = gbase + j;
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int idx = __shfl_sync(0xffffffffu, my_idx, lane0 + u);
-        if constexpr (ARG) e_u[u] = __shfl_sync(0xffffffffu, my_e, lane0 + u);
-        if constexpr (HAS_W) w_u[u] = __shfl_sync(0xffffffffu, my_w, lane0 + u);
+        if constexpr (ARG || HEADS) e_u[u] = __shfl_sync(0xffffffffu, my_e, lane0 + u);
+        if constexpr (HEADS) w_u[u] = vact ? DType<T>::to_f(whead[(int64_t)e_u[u] * p.H]) : 0.f;
+        else if constexpr (HAS_W) w_u[u] = __shfl_sync(0xffffffffu, my_w, lane0 + u);
         if (vact) val[u] = ld_vec<VB>(gather_addr(xcol, xcol2, x2f, (unsigned)idx, ldx));
       }
       // rows ascend: the batch's last row equal to cur_row means no boundary inside it
@@ -504,9 +517,12 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
       const int row_u = __shfl_sync(0xffffffffu, my_row, src_lane);
       int e1 = 0;
       float w1 = 0.f;
-      if constexpr (ARG) e1 = __shfl_sync(0xffffffffu, my_e, src_lane);
-      if constexpr (HAS_W) w1 = __shfl_sync(0xffffffffu, my_w, src_lane);
+      if constexpr (ARG || HEADS) e1 = __shfl_sync(0xffffffffu, my_e, src_lane);
+      if constexpr (HAS_W && !HEADS) w1 = __shfl_sync(0xffffffffu, my_w, src_lane);
       if (slot < rem) {
+        if constexpr (HEADS) {
+          if (vact) w1 = DType<T>::to_f(whead[(int64_t)e1 * p.H]);
+        }
         Words<VB> val1;
         if (vact) val1 = ld_vec<VB>(gather_addr(xcol, xcol2, x2f, (unsigned)idx, ldx));
         if (row_u != cur_row) {
@@ -540,8 +556,9 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
 // memory; the warps then read records with broadcast LDS instead of per-tile global loads and
 // shuffles.  No warp-synchronous operation is left in the loop, so every worker follows its own
 // row boundaries without dragging the other workers of its warp through the slow path.
-template <typename T, int VB, int RED, bool ARG, bool HAS_W, int U>
-__global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMinBlocks - 1 : kSegMinBlocks)
+template <typename T, int VB, int RED, bool ARG, bool HAS_W, int U, bool HEADS = false>
+__global__ void __launch_bounds__(kSegThreads, HEADS ? kSegMinBlocksHeads
+                                              : (ARG || sizeof(T) == 2) ? kSegMinBlocks - 1 : kSegMinBlocks)
     segreduce_staged_kernel(const SegParams p) {
   asm volatile("griddepcontrol.launch_dependents;");  // see segreduce_kernel
   constexpr int EPV = VB / (int)sizeof(T);
@@ -562,8 +579,9 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
   int* s_row = reinterpret_cast<int*>(smem_raw + 128);
   int* s_idx = s_row + cap;                       // used when p.gidx
-  int* s_e = s_idx + (p.gidx ? cap : 0);          // used when ARG and a separate eid array
-  const bool sep_e = ARG && p.eid && p.eid != p.gidx;
+  int* s_e = s_idx + (p.gidx ? cap : 0);          // used when ARG (or HEADS) and a separate eid array
+  const bool sep_e = (ARG || HEADS) && p.eid && p.eid != p.gidx;
+  constexpr bool W_SLAB = HAS_W && !HEADS;        // per-head weights are gathered, not staged
   T* s_w = reinterpret_cast<T*>(s_e + (sep_e ? cap : 0));
 
   const bool tma = p.tma_ok && (n % 8 == 0);
@@ -572,12 +590,12 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
     __syncthreads();
     if (threadIdx.x == 0) {
       uint32_t bytes = (uint32_t)n * 4u * (1u + (p.gidx ? 1u : 0u) + (sep_e ? 1u : 0u));
-      if (HAS_W) bytes += (uint32_t)n * (uint32_t)sizeof(T);
+      if (W_SLAB) bytes += (uint32_t)n * (uint32_t)sizeof(T);
       mbar_expect_tx(bar, bytes);
       bulk_g2s(s_row, p.erow + e0, (uint32_t)n * 4u, bar);
       if (p.gidx) bulk_g2s(s_idx, p.gidx + e0, (uint32_t)n * 4u, bar);
       if (sep_e) bulk_g2s(s_e, p.eid + e0, (uint32_t)n * 4u, bar);
-      if (HAS_W) bulk_g2s(s_w, static_cast<const T*>(p.w) + e0, (uint32_t)n * (uint32_t)sizeof(T), bar);
+      if (W_SLAB) bulk_g2s(s_w, static_cast<const T*>(p.w) + e0, (uint32_t)n * (uint32_t)sizeof(T), bar);
     }
     mbar_wait(bar, 0);
   } else {  // unaligned tail slab (or unaligned caller arrays): plain cooperative copy
@@ -585,7 +603,7 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
       s_row[i] = __ldg(p.erow + e0 + i);
       if (p.gidx) s_idx[i] = __ldg(p.gidx + e0 + i);
       if (sep_e) s_e[i] = __ldg(p.eid + e0 + i);
-      if (HAS_W) s_w[i] = static_cast<const T*>(p.w)[e0 + i];
+      if (W_SLAB) s_w[i] = static_cast<const T*>(p.w)[e0 + i];
     }
     __syncthreads();
   }
@@ -610,7 +628,8 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
   const int* ep = (sep_e ? s_e : s_idx) + soff;
   const T* wp = s_w + soff;
   const bool has_idx = p.gidx != nullptr;
-  const bool e_is_k = ARG && !sep_e && !(p.eid && p.eid == p.gidx);  // eid == NULL: edge id = k
+  const bool e_is_k = (ARG || HEADS) && !sep_e && !(p.eid && p.eid == p.gidx);  // eid == NULL: edge id = k
+  const T* whead = HEADS ? static_cast<const T*>(p.w) + (v * EPV) / p.head_c : nullptr;
 
   Accum<T, VB, RED, HAS_W> acc;
   int ae[ARG ? EPV : 1];
@@ -638,10 +657,12 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
   int t = 0;
   for (; t + U <= nv; t += U) {
     Words<VB> val[U];
+    float wh[HEADS ? U : 1];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int idx = has_idx ? idxp[t + u] : (int)(k0 + t + u);
       val[u] = ld_vec<VB>(gather_addr(xcol, xcol2, x2f, (unsigned)idx, ldx));
+      if constexpr (HEADS) wh[u] = DType<T>::to_f(whead[(int64_t)(e_is_k ? (int)(k0 + t + u) : ep[t + u]) * p.H]);
     }
     // rows ascend: the batch's last row equal to cur_row means no boundary inside it
     const bool simple = rowp[t + U - 1] == cur_row;
@@ -654,7 +675,8 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
       int e1 = 0;
       float w1 = 0.f;
       if constexpr (ARG) e1 = e_is_k ? (int)(k0 + t + u) : ep[t + u];
-      if constexpr (HAS_W) w1 = DType<T>::to_f(wp[t + u]);
+      if constexpr (HEADS) w1 = wh[HEADS ? u : 0];
+      else if constexpr (HAS_W) w1 = DType<T>::to_f(wp[t + u]);
       accumulate<T, VB, RED, ARG, HAS_W>(acc, ae, val[u], e1, w1);
     }
   }
@@ -667,7 +689,8 @@ __global__ void __launch_bounds__(kSegThreads, (ARG || sizeof(T) == 2) ? kSegMin
     int e1 = 0;
     float w1 = 0.f;
     if constexpr (ARG) e1 = e_is_k ? (int)(k0 + t) : ep[t];
-    if constexpr (HAS_W) w1 = DType<T>::to_f(wp[t]);
+    if constexpr (HEADS) w1 = DType<T>::to_f(whead[(int64_t)(e_is_k ? (int)(k0 + t) : ep[t]) * p.H]);
+    else if constexpr (HAS_W) w1 = DType<T>::to_f(wp[t]);
     accumulate<T, VB, RED, ARG, HAS_W>(acc, ae, val1, e1, w1);
   }
   if (nv > 0) {
@@ -860,23 +883,25 @@ static int64_t seg_staged_bytes(const SegParams& p, int es, bool arg, bool has_w
   return cap * 4 * (1 + (p.gidx ? 1 : 0) + (sep_e ? 1 : 0)) + (has_w ? cap * es : 0);
 }
 
-template <typename T, int VB, int RED, bool ARG, bool HAS_W>
+template <typename T, int VB, int RED, bool ARG, bool HAS_W, bool HEADS = false>
 static int launch_seg(const SegParams& p, cudaStream_t s) {
-  constexpr int U = (GNO_SEG_INFLIGHT / VB) > 16 ? 16 : (GNO_SEG_INFLIGHT / VB);
+  constexpr int U0 = (GNO_SEG_INFLIGHT / VB) > 16 ? 16 : (GNO_SEG_INFLIGHT / VB);
+  // per-head weights add a gathered value per unrolled edge: half the batch keeps them in registers
+  constexpr int U = (HEADS && U0 > 1) ? U0 / 2 : U0;
   const int64_t workers = p.n_chunks * p.ncoltiles;
   const int64_t warps = ceil_div(workers, 32 / p.G);
   const int64_t blocks = ceil_div(warps, kSegWarps);
   static const int carve = getenv("GNO_SEG_CARVEOUT") ? atoi(getenv("GNO_SEG_CARVEOUT")) : -1;
   if (carve >= 0) {
-    GNO_CUDA(cudaFuncSetAttribute(segreduce_staged_kernel<T, VB, RED, ARG, HAS_W, U>,
+    GNO_CUDA(cudaFuncSetAttribute(segreduce_staged_kernel<T, VB, RED, ARG, HAS_W, U, HEADS>,
                                   cudaFuncAttributePreferredSharedMemoryCarveout, carve));
   }
   if (blocks > 0 && p.staged) {
-    const size_t smem = 128 + (size_t)seg_staged_bytes(p, (int)sizeof(T), ARG, HAS_W);
-    segreduce_staged_kernel<T, VB, RED, ARG, HAS_W, U><<<(unsigned)blocks, kSegThreads, smem, s>>>(p);
+    const size_t smem = 128 + (size_t)seg_staged_bytes(p, (int)sizeof(T), ARG || HEADS, HAS_W && !HEADS);
+    segreduce_staged_kernel<T, VB, RED, ARG, HAS_W, U, HEADS><<<(unsigned)blocks, kSegThreads, smem, s>>>(p);
     GNO_LAUNCHED("segreduce_staged_kernel");
   } else if (blocks > 0) {
-    segreduce_kernel<T, VB, RED, ARG, HAS_W, U><<<(unsigned)blocks, kSegThreads, 0, s>>>(p);
+    segreduce_kernel<T, VB, RED, ARG, HAS_W, U, HEADS><<<(unsigned)blocks, kSegThreads, 0, s>>>(p);
     GNO_LAUNCHED("segreduce_kernel");
   }
   const int64_t quads = (p.F + 3) / 4;
@@ -911,6 +936,7 @@ static int dispatch_red(const SegParams& p, int reduce, bool /*with_arg*/, bool 
   switch (reduce) {
     case GNO_SUM:
     case GNO_MEAN:
+      if (p.H > 0) return launch_seg<T, VB, GNO_SUM, false, true, true>(p, s);
       return has_w ? launch_seg<T, VB, GNO_SUM, false, true>(p, s)
                    : launch_seg<T, VB, GNO_SUM, false, false>(p, s);
     case GNO_MUL:
@@ -940,6 +966,74 @@ static int dispatch_vb(const SegParams& p, int vb, int reduce, bool with_arg, bo
 }
 
 static int dtype_size(int dtype) { return dtype == GNO_F32 ? 4 : 2; }
+
+// ---- per-edge, per-head dot product (gradient of the per-head weights) ----------------------
+//   ga[eid[k] * H + h] = sum_c go[erow[k], h*C + c] * x[gidx[k], h*C + c]
+// One thread per (sorted edge, head); the H threads of an edge read the two rows whole.  Edges
+// arrive dst-sorted, so consecutive edges share their go row: it is read from DRAM once per row
+// and from L1 for the rest of the row's edges.  fp32 accumulation, one rounding.
+template <typename T, int VB>
+__global__ void __launch_bounds__(256) edge_head_dot_kernel(const int32_t* __restrict__ erow,
+                                                            const int32_t* __restrict__ gidx,
+                                                            const int32_t* __restrict__ eid,
+                                                            const char* __restrict__ x,
+                                                            const char* __restrict__ go, T* __restrict__ ga,
+                                                            int64_t total, int H, int64_t row_bytes,
+                                                            int nvh, bool narrow) {
+  constexpr int EPV = VB / (int)sizeof(T);
+  const int64_t t = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  if (t >= total) return;
+  const int64_t k = narrow ? (int64_t)((uint32_t)t / (uint32_t)H) : t / H;
+  const int h = (int)(t - k * H);
+  const int64_t row = __ldg(erow + k);
+  const int64_t s = gidx ? (int64_t)__ldg(gidx + k) : k;
+  const int64_t e = eid ? (int64_t)__ldg(eid + k) : k;
+  const char* xp = x + s * row_bytes + (int64_t)h * nvh * VB;
+  const char* gp = go + row * row_bytes + (int64_t)h * nvh * VB;
+  float acc = 0.f;
+  for (int j = 0; j < nvh; ++j) {
+    const Words<VB> a = ld_vec<VB>(xp + j * VB);
+    const Words<VB> b = ld_vec<VB>(gp + j * VB);
+#pragma unroll
+    for (int i = 0; i < EPV; ++i) acc = fmaf(elem<T, VB>(b, i), elem<T, VB>(a, i), acc);
+  }
+  ga[e * H + h] = DType<T>::from_f(acc);
+}
+
+// Widest vector (16/8/4/2 bytes) that divides one head's bytes and the alignment `a`.
+static int head_vector_bytes(int64_t head_bytes, uintptr_t a, int es) {
+  int vb = 16;
+  while (vb > es && ((a % vb) != 0 || head_bytes % vb != 0)) vb >>= 1;
+  return vb;
+}
+
+template <typename T>
+static int launch_edge_head_dot(const gno_csr* g, const void* x, const void* go, void* ga, int64_t H,
+                                int64_t F, cudaStream_t s) {
+  const int es = (int)sizeof(T);
+  const int64_t total = g->E * H;
+  if (total == 0 || F == 0) return GNO_OK;
+  const int vb = head_vector_bytes(F / H * es, (uintptr_t)x | (uintptr_t)go, es);
+  const int nvh = (int)(F / H * es / vb);
+  const unsigned blocks = (unsigned)ceil_div(total, 256);
+  const bool narrow = total < (int64_t(1) << 32);
+  const char* xc = static_cast<const char*>(x);
+  const char* gc = static_cast<const char*>(go);
+  T* out = static_cast<T*>(ga);
+  switch (vb) {
+    case 16: edge_head_dot_kernel<T, 16><<<blocks, 256, 0, s>>>(g->erow, g->gidx, g->eid, xc, gc, out, total, (int)H, F * es, nvh, narrow); break;
+    case 8: edge_head_dot_kernel<T, 8><<<blocks, 256, 0, s>>>(g->erow, g->gidx, g->eid, xc, gc, out, total, (int)H, F * es, nvh, narrow); break;
+    case 4: edge_head_dot_kernel<T, 4><<<blocks, 256, 0, s>>>(g->erow, g->gidx, g->eid, xc, gc, out, total, (int)H, F * es, nvh, narrow); break;
+    default:
+      if constexpr (sizeof(T) == 2) {
+        edge_head_dot_kernel<T, 2><<<blocks, 256, 0, s>>>(g->erow, g->gidx, g->eid, xc, gc, out, total, (int)H, F * es, nvh, narrow);
+        break;
+      }
+      return fail(GNO_ERR_INVALID, "gno_edge_head_dot: bad vector width %d", vb);
+  }
+  GNO_LAUNCHED("edge_head_dot_kernel");
+  return GNO_OK;
+}
 
 }  // namespace gno
 
@@ -972,10 +1066,13 @@ int gno_segment_reduce(const gno_csr* g, const void* x, int64_t x_rows, int64_t 
                                 accumulate, wsp, ws_bytes, stream);
 }
 
-int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int64_t ldx, const void* x2,
-                           int64_t x2_rows, const void* w, void* out, int64_t ldo, int64_t* arg,
-                           int64_t arg_fill, int64_t F, int dtype, int reduce, int accumulate, void* wsp,
-                           size_t ws_bytes, gno_stream_t stream) {
+}  // extern "C"
+
+// heads > 0: per-head weights (gno_segment_reduce_heads), w is [*, heads] read through g->eid.
+static int segment_reduce_impl(const gno_csr* g, const void* x, int64_t x_rows, int64_t ldx, const void* x2,
+                               int64_t x2_rows, const void* w, void* out, int64_t ldo, int64_t* arg,
+                               int64_t arg_fill, int64_t F, int dtype, int reduce, int accumulate, void* wsp,
+                               size_t ws_bytes, gno_stream_t stream, int64_t heads) {
   cudaStream_t s = (cudaStream_t)stream;
   GNO_CHECK_ARG(x2 == nullptr || (x2_rows >= 0 && x_rows + x2_rows < (int64_t(1) << 31)),
                 "gno_segment_reduce_two: x_rows + x2_rows must stay below 2^31");
@@ -1012,6 +1109,7 @@ int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int6
   int vb = 16;
   while (vb > es && (ax % vb) != 0) vb >>= 1;
   while (vb > es && (F * es) % vb != 0 && ceil_div(F * es, vb) * vb > ldx * es) vb >>= 1;
+  if (heads > 0) vb = head_vector_bytes(F / heads * es, (uintptr_t)vb, es);  // a vector stays inside one head
   const uintptr_t ao = (uintptr_t)out | (uintptr_t)(ldo * es) | (uintptr_t)(F * es);
 
   SegParams p;
@@ -1046,6 +1144,8 @@ int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int6
   p.G = G;
   p.mean = (reduce == GNO_MEAN);
   p.accumulate = accumulate ? 1 : 0;
+  p.H = (int)heads;
+  p.head_c = heads > 0 ? (int)(F / heads) : 0;
   p.part_val = nullptr;
   p.part_arg = nullptr;
   if (p.n_chunks > 0) {
@@ -1060,11 +1160,12 @@ int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int6
   const bool has_w = (w != nullptr);
   {
     const bool argv = (reduce == GNO_MIN || reduce == GNO_MAX);
-    const uintptr_t al = (uintptr_t)g->erow | (uintptr_t)g->gidx | (uintptr_t)(argv ? g->eid : nullptr) |
-                         (uintptr_t)w;
+    const bool hd = heads > 0;
+    const uintptr_t al = (uintptr_t)g->erow | (uintptr_t)g->gidx | (uintptr_t)(argv || hd ? g->eid : nullptr) |
+                         (uintptr_t)(hd ? nullptr : w);
     p.tma_ok = (al % 16) == 0;
     static const int staged_env = getenv("GNO_SEG_STAGED") ? atoi(getenv("GNO_SEG_STAGED")) : 1;
-    p.staged = staged_env && seg_staged_bytes(p, es, argv, has_w) <= 24 * 1024;
+    p.staged = staged_env && seg_staged_bytes(p, es, argv || hd, has_w && !hd) <= 24 * 1024;
   }
   switch (dtype) {
     case GNO_F32: return dispatch_vb<float>(p, vb, reduce, with_arg, has_w, s);
@@ -1072,6 +1173,50 @@ int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int6
     case GNO_BF16: return dispatch_vb<__nv_bfloat16>(p, vb, reduce, with_arg, has_w, s);
   }
   return fail(GNO_ERR_INVALID, "gno_segment_reduce: unknown dtype %d", dtype);
+}
+
+extern "C" {
+
+int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int64_t ldx, const void* x2,
+                           int64_t x2_rows, const void* w, void* out, int64_t ldo, int64_t* arg,
+                           int64_t arg_fill, int64_t F, int dtype, int reduce, int accumulate, void* wsp,
+                           size_t ws_bytes, gno_stream_t stream) {
+  return segment_reduce_impl(g, x, x_rows, ldx, x2, x2_rows, w, out, ldo, arg, arg_fill, F, dtype, reduce,
+                             accumulate, wsp, ws_bytes, stream, 0);
+}
+
+int gno_segment_reduce_heads(const gno_csr* g, const void* x, int64_t x_rows, const void* alpha, int64_t H,
+                             void* out, int64_t F, int dtype, void* ws, size_t ws_bytes, gno_stream_t stream) {
+  GNO_CHECK_ARG(dtype == GNO_F32 || dtype == GNO_F16 || dtype == GNO_BF16,
+                "gno_segment_reduce_heads: unknown dtype %d", dtype);
+  GNO_CHECK_ARG(H > 0 && H < (int64_t(1) << 20) && F >= 0 && F % H == 0 && x_rows >= 0,
+                "gno_segment_reduce_heads: bad sizes H=%lld F=%lld x_rows=%lld", (long long)H, (long long)F,
+                (long long)x_rows);
+  GNO_CHECK_ARG(g == nullptr || g->E == 0 || F == 0 || alpha != nullptr, "gno_segment_reduce_heads: alpha is NULL");
+  return segment_reduce_impl(g, x, x_rows, F, nullptr, 0, alpha, out, F, nullptr, 0, F, dtype, GNO_SUM, 0, ws,
+                             ws_bytes, stream, H);
+}
+
+int gno_edge_head_dot(const gno_csr* g, const void* x, int64_t x_rows, const void* grad_out, int64_t H,
+                      int64_t F, void* grad_alpha, int dtype, gno_stream_t stream) {
+  GNO_CHECK_ARG(g != nullptr, "gno_edge_head_dot: graph is NULL");
+  GNO_CHECK_ARG(dtype == GNO_F32 || dtype == GNO_F16 || dtype == GNO_BF16, "gno_edge_head_dot: unknown dtype %d",
+                dtype);
+  GNO_CHECK_ARG(H > 0 && H < (int64_t(1) << 20) && F >= 0 && F % H == 0 && x_rows >= 0 && g->N >= 0 &&
+                    g->E >= 0 && g->E < (int64_t(1) << 31),
+                "gno_edge_head_dot: bad sizes H=%lld F=%lld x_rows=%lld E=%lld", (long long)H, (long long)F,
+                (long long)x_rows, (long long)g->E);
+  if (g->E == 0 || F == 0) return GNO_OK;
+  GNO_CHECK_ARG(g->erow && x && grad_out && grad_alpha, "gno_edge_head_dot: NULL buffer");
+  const int es = dtype_size(dtype);
+  GNO_CHECK_ARG((((uintptr_t)x | (uintptr_t)grad_out | (uintptr_t)grad_alpha) % es) == 0,
+                "gno_edge_head_dot: buffers not aligned to the element size");
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (dtype) {
+    case GNO_F32: return launch_edge_head_dot<float>(g, x, grad_out, grad_alpha, H, F, s);
+    case GNO_F16: return launch_edge_head_dot<__half>(g, x, grad_out, grad_alpha, H, F, s);
+    default: return launch_edge_head_dot<__nv_bfloat16>(g, x, grad_out, grad_alpha, H, F, s);
+  }
 }
 
 }  // extern "C"

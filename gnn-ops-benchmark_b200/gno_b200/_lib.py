@@ -5,7 +5,7 @@ import fails loudly — the product path is the CUDA library or nothing.
 """
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_int, c_int64, c_size_t, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_int, c_int64, c_size_t, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libgno_b200.so")
@@ -67,6 +67,15 @@ PROTOTYPES = {
     "gno_segment_reduce_two": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_int64, c_void_p, c_int64, c_void_p,
                                        c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int, c_int,
                                        c_int, c_void_p, c_size_t, c_void_p]),
+    "gno_segment_reduce_heads": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_int64, c_void_p,
+                                         c_int64, c_int, c_void_p, c_size_t, c_void_p]),
+    "gno_edge_head_dot": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_int64, c_int64, c_void_p,
+                                  c_int, c_void_p]),
+    "gno_segment_softmax_workspace": (c_int, [POINTER(gno_csr), c_int64, POINTER(c_size_t)]),
+    "gno_segment_softmax": (c_int, [POINTER(gno_csr), c_void_p, c_void_p, c_int64, c_int64, c_double, c_void_p,
+                                    c_int, c_void_p, c_size_t, c_void_p]),
+    "gno_segment_softmax_backward": (c_int, [POINTER(gno_csr), c_void_p, c_void_p, c_void_p, c_int64, c_int64,
+                                             c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
     "gno_segment_reduce_int": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_int64, c_void_p,
                                        c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
     "gno_segment_reduce_lastdim": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_int64, c_int64,

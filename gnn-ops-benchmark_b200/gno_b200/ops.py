@@ -76,6 +76,8 @@ def clear_caches():
     _memo_store.clear()
     _pad_store.clear()
     _fast_calls.clear()
+    from . import attention  # imports this module: bound at call time
+    attention._sorted_alpha.clear()
 
 
 # ------------------------------------------------------------ segment reduce --

@@ -205,6 +205,59 @@ int gno_segment_reduce_two(const gno_csr* g, const void* x, int64_t x_rows, int6
                            size_t ws_bytes, gno_stream_t stream);
 
 /*
+ * Multi-head attention aggregation (GATv2's message passing, PyG
+ * GATv2Conv.message + aggregate):
+ *   out[i, h*C + c] = sum over sorted edges k in row i of
+ *                     alpha[eid[k] * H + h] * x[gidx[k], h*C + c]
+ * x [x_rows, F] and out [N, F] contiguous, F = H*C; alpha [*, H] in x's dtype,
+ * read through the ORIGINAL edge id eid[k] (NULL = k), so a dst-sorted plan and
+ * the src-sorted plan of the transposed aggregation (the backward w.r.t. x)
+ * read the same tensor.  The segment-reduce kernel with a per-head weight: a
+ * gathered vector covers columns of one head only.  With H = 1 the arithmetic
+ * is gno_segment_reduce's with w[k] = alpha[eid[k]], in the same order.
+ * ws >= gno_segment_reduce_workspace(g, F, dtype, GNO_SUM, 0) bytes.
+ */
+int gno_segment_reduce_heads(const gno_csr* g, const void* x, int64_t x_rows,
+                             const void* alpha, int64_t H, void* out, int64_t F,
+                             int dtype, void* ws, size_t ws_bytes,
+                             gno_stream_t stream);
+
+/*
+ * Per-edge, per-head dot product (the gradient w.r.t. alpha of
+ * gno_segment_reduce_heads), over a dst-sorted plan:
+ *   grad_alpha[eid[k] * H + h] = sum_c grad_out[erow[k], h*C + c] * x[gidx[k], h*C + c]
+ * x [x_rows, F], grad_out [N, F] contiguous, F = H*C; fp32 accumulation.  Edges
+ * the plan dropped are not written.
+ */
+int gno_edge_head_dot(const gno_csr* g, const void* x, int64_t x_rows,
+                      const void* grad_out, int64_t H, int64_t F,
+                      void* grad_alpha, int dtype, gno_stream_t stream);
+
+/*
+ * Segment softmax over destination rows (torch_geometric.utils.softmax of PyG
+ * 2.0.2, GATv2REG's attention normalisation), H heads per edge:
+ *   m[i, h] = max of the row's logits (torch_scatter rule: start at the dtype's
+ *             lowest finite value, strictly greater wins, NaN never wins, no
+ *             winner -> 0)
+ *   out[e, h] = exp(src[e, h] - m[dst[e], h]) / (sum over the row of exp(src - m) + eps)
+ * src / out [E, H] are in ORIGINAL edge order.  dst[e] = index[e] (int64, the
+ * index the plan was built from; edges outside [0, N) get 0), or index = NULL
+ * for a plan made by gno_plan_from_rowptr (original order = sorted order,
+ * E = g->E).  The plan's eid must be its perm (NULL with a rowptr plan).  fp32
+ * math, one rounding; atomic-free and bit-reproducible.  The backward writes
+ *   grad_src[e, h] = out[e, h] * (grad_out[e, h] - sum over the row of grad_out * out).
+ * ws >= gno_segment_softmax_workspace(g, H) bytes (both directions).
+ */
+int gno_segment_softmax_workspace(const gno_csr* g, int64_t H, size_t* bytes);
+int gno_segment_softmax(const gno_csr* g, const void* src, const int64_t* index,
+                        int64_t E, int64_t H, double eps, void* out, int dtype,
+                        void* ws, size_t ws_bytes, gno_stream_t stream);
+int gno_segment_softmax_backward(const gno_csr* g, const void* out,
+                                 const void* grad_out, const int64_t* index,
+                                 int64_t E, int64_t H, void* grad_src, int dtype,
+                                 void* ws, size_t ws_bytes, gno_stream_t stream);
+
+/*
  * Integer form (int32 / int64 values, exact int64 accumulation): torch_scatter.scatter on
  * integer tensors — PyG's TopKPooling / to_dense_batch count nodes per graph with
  * scatter_add(batch.new_ones(n), batch, dim=0) (graph_benchmark/models/ptg_models.py:165-172).
