@@ -26,7 +26,7 @@
 #include <cstdlib>
 #include <type_traits>
 
-#include "common.cuh"
+#include "segreduce.cuh"
 
 namespace gno {
 
@@ -46,38 +46,6 @@ constexpr int kSegMinBlocksHeads = 6;
 constexpr int kSegMinBlocksHeadsWide = 5;
 constexpr int kNoArg = INT_MAX;
 
-struct SegParams {
-  const int32_t* gidx;
-  const int32_t* eid;
-  const int32_t* erow;
-  const void* x;
-  const void* x2;      // second gather base (gno_segment_reduce_two): gather ids >= x2_first read row id - x2_first of x2
-  const void* w;
-  void* out;
-  int64_t* arg;
-  float* part_val;    // [2 * n_chunks, F] fp32 partials of rows cut by a chunk boundary
-  int32_t* part_arg;  // [2 * n_chunks, F]
-  const int64_t* rowptr;
-  const int32_t* srow;
-  const int32_t* zrow;
-  int64_t N, E, n_chunks, n_span, n_empty;
-  int64_t F;
-  int64_t Fp;  // row stride of the partial buffers: F rounded up to 8 elements
-  int64_t ldx_bytes, ldo_bytes;
-  int64_t arg_fill;
-  int chunk_len;  // edges per worker
-  int nvec;       // vectors per row
-  int ncoltiles;  // column tiles of 32 vectors
-  int G;          // lanes per worker (power of two; 32 when ncoltiles > 1)
-  int mean;       // divide by max(row length, 1)
-  int accumulate;
-  int vec_out;    // out rows are aligned for VB-byte vector stores and F*s is a multiple of VB
-  int tma_ok;     // edge-record arrays are 16-byte aligned (bulk copies allowed)
-  int staged;     // use the TMA-staged kernel (record slab of a CTA fits the shared-memory budget)
-  unsigned x2_first;  // 0xffffffff when there is no second base (no gather id reaches it)
-  int H;              // per-head weights (gno_segment_reduce_heads): w is [*, H], read at w[eid * H + h]
-  int head_c;         // columns per head; a gathered vector never straddles two heads
-};
 
 // Address of row `idx` of the gather source: two bases, one compare and a select (xcol2 is
 // pre-offset by -x2_first rows, so both forms add idx * ldx).
@@ -86,86 +54,6 @@ __device__ __forceinline__ const char* gather_addr(const char* xcol, const char*
   return (idx >= x2_first ? xcol2 : xcol) + (uint64_t)idx * ldx;
 }
 
-template <int VB>
-struct Words {
-  static constexpr int n = VB >= 4 ? VB / 4 : 1;
-  uint32_t w[n];
-};
-
-template <int VB>
-__device__ __forceinline__ Words<VB> ld_vec(const char* p) {
-  Words<VB> r;
-  if constexpr (VB == 16) {
-    const uint4 q = __ldg(reinterpret_cast<const uint4*>(p));
-    r.w[0] = q.x; r.w[1] = q.y; r.w[2] = q.z; r.w[3] = q.w;
-  } else if constexpr (VB == 8) {
-    const uint2 q = __ldg(reinterpret_cast<const uint2*>(p));
-    r.w[0] = q.x; r.w[1] = q.y;
-  } else if constexpr (VB == 4) {
-    r.w[0] = __ldg(reinterpret_cast<const uint32_t*>(p));
-  } else {
-    r.w[0] = __ldg(reinterpret_cast<const unsigned short*>(p));
-  }
-  return r;
-}
-template <int VB>
-__device__ __forceinline__ void st_vec(char* p, const Words<VB>& r) {
-  if constexpr (VB == 16) {
-    *reinterpret_cast<uint4*>(p) = make_uint4(r.w[0], r.w[1], r.w[2], r.w[3]);
-  } else if constexpr (VB == 8) {
-    *reinterpret_cast<uint2*>(p) = make_uint2(r.w[0], r.w[1]);
-  } else if constexpr (VB == 4) {
-    *reinterpret_cast<uint32_t*>(p) = r.w[0];
-  } else {
-    *reinterpret_cast<unsigned short*>(p) = (unsigned short)r.w[0];
-  }
-}
-
-template <typename T>
-__device__ __forceinline__ float bits_to_f(uint32_t b);
-template <>
-__device__ __forceinline__ float bits_to_f<float>(uint32_t b) { return __uint_as_float(b); }
-template <>
-__device__ __forceinline__ float bits_to_f<__half>(uint32_t b) {
-  return __half2float(__ushort_as_half((unsigned short)b));
-}
-template <>
-__device__ __forceinline__ float bits_to_f<__nv_bfloat16>(uint32_t b) {
-  return __uint_as_float(b << 16);
-}
-template <typename T>
-__device__ __forceinline__ uint32_t f_to_bits(float f);
-template <>
-__device__ __forceinline__ uint32_t f_to_bits<float>(float f) { return __float_as_uint(f); }
-template <>
-__device__ __forceinline__ uint32_t f_to_bits<__half>(float f) {
-  return __half_as_ushort(__float2half_rn(f));
-}
-template <>
-__device__ __forceinline__ uint32_t f_to_bits<__nv_bfloat16>(float f) {
-  return __bfloat16_as_ushort(__float2bfloat16_rn(f));
-}
-
-template <typename T, int VB>
-__device__ __forceinline__ float elem(const Words<VB>& r, int i) {
-  if constexpr (sizeof(T) == 4) {
-    return bits_to_f<T>(r.w[i]);
-  } else {
-    return bits_to_f<T>((r.w[i >> 1] >> ((i & 1) * 16)) & 0xffffu);
-  }
-}
-template <typename T, int VB>
-__device__ __forceinline__ void set_elem(Words<VB>& r, int i, float f) {
-  if constexpr (sizeof(T) == 4) {
-    r.w[i] = f_to_bits<T>(f);
-  } else {
-    const uint32_t b = f_to_bits<T>(f) & 0xffffu;
-    if (i & 1)
-      r.w[i >> 1] |= b << 16;
-    else
-      r.w[i >> 1] = b;
-  }
-}
 
 template <typename T, int RED>
 __device__ __forceinline__ float red_init() {
@@ -883,6 +771,36 @@ static int64_t seg_staged_bytes(const SegParams& p, int es, bool arg, bool has_w
   return cap * 4 * (1 + (p.gidx ? 1 : 0) + (sep_e ? 1 : 0)) + (has_w ? cap * es : 0);
 }
 
+// The finish pass behind a chunk kernel (after_kernel: it was launched just before, so this one
+// may start early under programmatic stream serialization).
+template <typename T, int RED, bool ARG>
+static int launch_segfinish(const SegParams& p, bool after_kernel, cudaStream_t s) {
+  const int64_t quads = (p.F + 3) / 4;
+  const int64_t per_empty = seg_fill16(p, (int)sizeof(T), ARG) ? p.F / (16 / (int64_t)sizeof(T)) : quads;
+  const int64_t total = p.n_span * quads + (p.accumulate ? 0 : p.n_empty * per_empty);
+  if (total > 0) {
+    const int grid = (int)imin64(ceil_div(total, 256), (int64_t)kNumSMs * 16);
+    static const int pdl_env = getenv("GNO_SEG_PDL") ? atoi(getenv("GNO_SEG_PDL")) : 1;
+    if (after_kernel && pdl_env) {
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3((unsigned)grid);
+      cfg.blockDim = dim3(256);
+      cfg.dynamicSmemBytes = 0;
+      cfg.stream = s;
+      cudaLaunchAttribute at[1];
+      at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+      at[0].val.programmaticStreamSerializationAllowed = 1;
+      cfg.attrs = at;
+      cfg.numAttrs = 1;
+      GNO_CUDA(cudaLaunchKernelEx(&cfg, segfinish_kernel<T, RED, ARG>, p));
+    } else {
+      segfinish_kernel<T, RED, ARG><<<grid, 256, 0, s>>>(p);
+    }
+    GNO_LAUNCHED("segfinish_kernel");
+  }
+  return GNO_OK;
+}
+
 template <typename T, int VB, int RED, bool ARG, bool HAS_W, bool HEADS = false>
 static int launch_seg(const SegParams& p, cudaStream_t s) {
   constexpr int U0 = (GNO_SEG_INFLIGHT / VB) > 16 ? 16 : (GNO_SEG_INFLIGHT / VB);
@@ -904,30 +822,7 @@ static int launch_seg(const SegParams& p, cudaStream_t s) {
     segreduce_kernel<T, VB, RED, ARG, HAS_W, U, HEADS><<<(unsigned)blocks, kSegThreads, 0, s>>>(p);
     GNO_LAUNCHED("segreduce_kernel");
   }
-  const int64_t quads = (p.F + 3) / 4;
-  const int64_t per_empty = seg_fill16(p, (int)sizeof(T), ARG) ? p.F / (16 / (int64_t)sizeof(T)) : quads;
-  const int64_t total = p.n_span * quads + (p.accumulate ? 0 : p.n_empty * per_empty);
-  if (total > 0) {
-    const int grid = (int)imin64(ceil_div(total, 256), (int64_t)kNumSMs * 16);
-    static const int pdl_env = getenv("GNO_SEG_PDL") ? atoi(getenv("GNO_SEG_PDL")) : 1;
-    if (blocks > 0 && pdl_env) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3((unsigned)grid);
-      cfg.blockDim = dim3(256);
-      cfg.dynamicSmemBytes = 0;
-      cfg.stream = s;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      at[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = at;
-      cfg.numAttrs = 1;
-      GNO_CUDA(cudaLaunchKernelEx(&cfg, segfinish_kernel<T, RED, ARG>, p));
-    } else {
-      segfinish_kernel<T, RED, ARG><<<grid, 256, 0, s>>>(p);
-    }
-    GNO_LAUNCHED("segfinish_kernel");
-  }
-  return GNO_OK;
+  return launch_segfinish<T, RED, ARG>(p, blocks > 0, s);
 }
 
 template <typename T, int VB>
@@ -967,6 +862,14 @@ static int dispatch_vb(const SegParams& p, int vb, int reduce, bool with_arg, bo
 
 static int dtype_size(int dtype) { return dtype == GNO_F32 ? 4 : 2; }
 
+int seg_finish_sum(const SegParams& p, int dtype, bool after_kernel, cudaStream_t s) {
+  switch (dtype) {
+    case GNO_F32: return launch_segfinish<float, GNO_SUM, false>(p, after_kernel, s);
+    case GNO_F16: return launch_segfinish<__half, GNO_SUM, false>(p, after_kernel, s);
+    default: return launch_segfinish<__nv_bfloat16, GNO_SUM, false>(p, after_kernel, s);
+  }
+}
+
 // ---- per-edge, per-head dot product (gradient of the per-head weights) ----------------------
 //   ga[eid[k] * H + h] = sum_c go[erow[k], h*C + c] * x[gidx[k], h*C + c]
 // One thread per (sorted edge, head); the H threads of an edge read the two rows whole.  Edges
@@ -998,13 +901,6 @@ __global__ void __launch_bounds__(256) edge_head_dot_kernel(const int32_t* __res
     for (int i = 0; i < EPV; ++i) acc = fmaf(elem<T, VB>(b, i), elem<T, VB>(a, i), acc);
   }
   ga[e * H + h] = DType<T>::from_f(acc);
-}
-
-// Widest vector (16/8/4/2 bytes) that divides one head's bytes and the alignment `a`.
-static int head_vector_bytes(int64_t head_bytes, uintptr_t a, int es) {
-  int vb = 16;
-  while (vb > es && ((a % vb) != 0 || head_bytes % vb != 0)) vb >>= 1;
-  return vb;
 }
 
 template <typename T>

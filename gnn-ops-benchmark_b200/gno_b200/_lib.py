@@ -76,6 +76,13 @@ PROTOTYPES = {
                                     c_int, c_void_p, c_size_t, c_void_p]),
     "gno_segment_softmax_backward": (c_int, [POINTER(gno_csr), c_void_p, c_void_p, c_void_p, c_int64, c_int64,
                                              c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "gno_gatv2_logits": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64,
+                                 c_double, c_void_p, c_int, c_void_p]),
+    "gno_gatv2_logits_backward_workspace": (c_int, [POINTER(gno_csr), c_int64, c_int64, c_int, c_int,
+                                                    POINTER(c_size_t)]),
+    "gno_gatv2_logits_backward": (c_int, [POINTER(gno_csr), c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
+                                          c_int64, c_int64, c_double, c_void_p, c_void_p, c_int, c_void_p,
+                                          c_size_t, c_void_p]),
     "gno_segment_reduce_int": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_int64, c_void_p,
                                        c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
     "gno_segment_reduce_lastdim": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_int64, c_int64,

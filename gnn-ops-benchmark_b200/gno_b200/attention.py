@@ -1,14 +1,14 @@
-"""Graph attention on the fused path: the segment softmax of torch_geometric.utils.softmax and the
-multi-head attention-weighted aggregation of a GATv2 layer (GATv2REG, SURVEY.md §3), forward and
-backward, on the CUDA library (include/gno_b200.h: gno_segment_softmax, gno_segment_reduce_heads,
-gno_edge_head_dot).
+"""Graph attention on the fused path: the attention logits of a GATv2 layer, the segment softmax of
+torch_geometric.utils.softmax and the multi-head attention-weighted aggregation (GATv2REG,
+SURVEY.md §3), forward and backward, on the CUDA library (include/gno_b200.h: gno_gatv2_logits*,
+gno_segment_softmax, gno_segment_reduce_heads, gno_edge_head_dot).
 
-A GATv2 layer computes per-edge, per-head logits [E, H] with dense torch ops, normalises them over
+A GATv2 layer computes per-edge, per-head logits [E, H] with `gatv2_logits`, normalises them over
 each destination's incoming edges with `softmax`, and aggregates
     out[i, h, :] = sum_{e: dst[e] = i} alpha[e, h] * x[src[e], h, :]
-with `attention_aggregate`, without materialising the [E, H, C] messages.  Both ops use the cached
-dst-sorted plan of the destination index; the backward of the aggregation w.r.t. x is the same
-kernel on the cached src-sorted plan, so a training step builds two plans once and reuses them.
+with `attention_aggregate`, without materialising the [E, H, C] messages.  All three ops use the
+cached dst-sorted plan of the destination index; the backward passes that scatter to source nodes
+run on the cached src-sorted plan, so a training step builds two plans once and reuses them.
 """
 import collections
 import ctypes
@@ -218,3 +218,107 @@ def attention_aggregate(x, alpha, src, dst, dim_size):
     a2 = alpha.reshape(E, H).to(x.dtype).contiguous()
     out = _AttentionAggregate.apply(x2, a2, src.contiguous(), dst.contiguous(), dim_size)
     return out.view(dim_size, H, C)
+
+
+def _gatv2_backward(plan, gidx, own, other, att, g, H, slope, grad_own, grad_att):
+    """One backward pass of the logits along `plan`: grad_own (or None) and fp32 grad_att (or None)."""
+    F = own.size(1)
+    dev = own.device
+    csr = plan.csr(gidx, plan.perm)
+    nbytes = ctypes.c_size_t()
+    check(lib.gno_gatv2_logits_backward_workspace(ctypes.byref(csr), H, F, grad_own is not None,
+                                                  grad_att is not None, ctypes.byref(nbytes)))
+    ws = _workspace(nbytes.value, dev)
+    with _on_device(dev):
+        check(lib.gno_gatv2_logits_backward(ctypes.byref(csr), _ptr(own), _ptr(other), other.size(0), _ptr(att),
+                                            _ptr(g), H, F, slope, _ptr(grad_own), _ptr(grad_att),
+                                            ops._dtype_id(own), _ptr(ws), nbytes.value, _stream(dev)))
+
+
+class _GATv2Logits(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x_l, x_r, att, src, dst, H, slope):
+        E, F = src.numel(), x_l.size(1)
+        ctx.H, ctx.slope = H, slope
+        ctx.save_for_backward(x_l, x_r, att, src, dst)
+        if E == 0 or F == 0:  # nothing to sum: zeros, and zero gradients below
+            return torch.zeros((E, H), dtype=x_l.dtype, device=x_l.device)
+        out = torch.empty((E, H), dtype=x_l.dtype, device=x_l.device)
+        plan = plan_cache.get(dst, x_r.size(0))
+        csr = plan.csr(plan.sorted_ids(src), plan.perm)
+        with _on_device(x_l.device):
+            check(lib.gno_gatv2_logits(ctypes.byref(csr), _ptr(x_l), x_l.size(0), _ptr(x_r), _ptr(att), H, F, slope,
+                                       _ptr(out), ops._dtype_id(x_l), _stream(x_l.device)))
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_logits):
+        x_l, x_r, att, src, dst = ctx.saved_tensors
+        need_l, need_r, need_att = ctx.needs_input_grad[:3]
+        g = grad_logits.to(x_l.dtype).contiguous()
+        H, slope = ctx.H, ctx.slope
+        empty = src.numel() == 0 or x_l.size(1) == 0
+        new = torch.zeros_like if empty else torch.empty_like
+        grad_l = new(x_l) if need_l else None
+        grad_r = new(x_r) if need_r else None
+        grad_att = new(att, dtype=torch.float32) if need_att else None
+        if not empty and (need_r or need_att):
+            plan = plan_cache.get(dst, x_r.size(0))
+            _gatv2_backward(plan, plan.sorted_ids(src), x_r, x_l, att, g, H, slope, grad_r, grad_att)
+        if not empty and need_l:
+            plan_t = plan_cache.get(src, x_l.size(0))
+            _gatv2_backward(plan_t, plan_t.sorted_ids(dst), x_l, x_r, att, g, H, slope, grad_l, None)
+        if grad_att is not None:
+            grad_att = grad_att.to(att.dtype)
+        return grad_l, grad_r, grad_att, None, None, None, None
+
+
+def _heads_view(t, name, H, C):
+    """[N, H, C] or [N, H*C] -> [N, H*C] (checks H and C against att's)."""
+    if t.dim() == 3:
+        if t.size(1) != H or t.size(2) != C:
+            raise ValueError(f"gatv2_logits: {name} is [N, {t.size(1)}, {t.size(2)}], att [{H}, {C}]")
+    elif t.dim() != 2 or t.size(1) != H * C:
+        raise ValueError(f"gatv2_logits: {name} must be [N, {H}, {C}] or [N, {H * C}], got {tuple(t.shape)}")
+    return t.reshape(t.size(0), H * C).contiguous()
+
+
+def gatv2_logits(x_l, x_r, att, src, dst, negative_slope=0.2):
+    """logits[e, h] = sum_c att[h, c] * leaky_relu(x_l[src[e], h, c] + x_r[dst[e], h, c], negative_slope)
+    — PyG 2.0.2 GATv2Conv.message (x_i + x_j, leaky_relu, (x * att).sum(-1)) without the [E, H, C]
+    messages.
+
+    x_l [N_src, H, C] or [N_src, H*C]; x_r [N_dst, H, C] or [N_dst, H*C] (N_src != N_dst allowed);
+    att [H, C], [1, H, C] (GATv2Conv's parameter) or [H*C], cast to x_l's dtype; src / dst int64 [E].
+    Returns [E, H] in x_l's dtype, in the original edge order (what `softmax` consumes).  The sum
+    x_l + x_r is formed in fp32 from the stored values; fp32 math, one rounding.  An out-of-range
+    src or dst raises IndexError.  Differentiable w.r.t. x_l, x_r and att (x_l and x_r may be the
+    same tensor); the backward recomputes the sums and saves no [E, ...] tensor."""
+    ops._need_cuda(x_l, x_r, att, src, dst)
+    ops._dtype_id(x_l)
+    if x_r.dtype != x_l.dtype:
+        raise ValueError(f"gatv2_logits: x_l is {x_l.dtype}, x_r {x_r.dtype}")
+    for name, t in (("src", src), ("dst", dst)):
+        if t.dtype != torch.int64 or t.dim() != 1:
+            raise ValueError(f"gatv2_logits: {name} must be a 1-D int64 tensor")
+    E = src.numel()
+    if dst.numel() != E:
+        raise ValueError("gatv2_logits: src and dst differ in length")
+    if att.dim() == 3 and att.size(0) == 1:
+        H, C = att.size(1), att.size(2)
+    elif att.dim() == 2:
+        H, C = att.shape
+    elif att.dim() == 1 and (x_l.dim() == 3 or x_r.dim() == 3):
+        H, C = (x_l if x_l.dim() == 3 else x_r).shape[1:]
+    elif att.dim() == 1:
+        raise ValueError("gatv2_logits: a flat att needs x_l or x_r as [N, H, C] to know the heads")
+    else:
+        raise ValueError(f"gatv2_logits: att must be [H, C], [1, H, C] or [H*C], got {tuple(att.shape)}")
+    if H == 0 or att.numel() != H * C:
+        raise ValueError(f"gatv2_logits: att has {att.numel()} entries for {H} heads of {C}")
+    xl2 = _heads_view(x_l, "x_l", H, C)
+    xr2 = _heads_view(x_r, "x_r", H, C)
+    ops._check_range(src, xl2.size(0), "gatv2_logits: src")
+    ops._check_range(dst, xr2.size(0), "gatv2_logits: dst")
+    a2 = att.reshape(H * C).to(x_l.dtype).contiguous()
+    return _GATv2Logits.apply(xl2, xr2, a2, src.contiguous(), dst.contiguous(), H, float(negative_slope))

@@ -258,6 +258,43 @@ int gno_segment_softmax_backward(const gno_csr* g, const void* out,
                                  void* ws, size_t ws_bytes, gno_stream_t stream);
 
 /*
+ * GATv2 attention logits (PyG 2.0.2 GATv2Conv.message: leaky_relu(x_i + x_j),
+ * then (. * att).sum(-1)), over the dst-sorted plan of dst with gidx = src[perm]:
+ *   out[eid[k] * H + h] = sum_c att[h*C + c] *
+ *       leaky_relu(x_l[gidx[k], h*C + c] + x_r[erow[k], h*C + c], negative_slope)
+ * x_l [xl_rows, F], x_r [N, F], att [F] contiguous in `dtype`, F = H*C; out [E, H]
+ * in original edge order.  The sum z is formed in fp32 from the stored values;
+ * fp32 accumulation, one rounding.  E = 0 touches nothing.
+ */
+int gno_gatv2_logits(const gno_csr* g, const void* x_l, int64_t xl_rows,
+                     const void* x_r, const void* att, int64_t H, int64_t F,
+                     double negative_slope, void* out, int dtype,
+                     gno_stream_t stream);
+
+/*
+ * Backward of gno_gatv2_logits along one plan (grad_logits [E, H], original order):
+ *   grad_own[i, f] = att[f] * sum_{k in row i} grad_logits[eid[k]*H + h] * (z > 0 ? 1 : slope)
+ *   grad_att[f]    = sum over the plan's edges of grad_logits[eid[k]*H + h] * leaky_relu(z)
+ * with z = other[gidx[k], f] + own[i, f] in fp32 and h = f / C.  Run on the dst
+ * plan with own = x_r, other = x_l (gidx = src[perm]) for grad_x_r and grad_att, and
+ * on the src plan with own = x_l, other = x_r (gidx = dst[perm]) for grad_x_l.
+ * grad_own [N, F] in `dtype` (empty rows get 0) and grad_att fp32 [F] may each be
+ * NULL, not both.  No atomics: bit-reproducible.
+ * ws >= gno_gatv2_logits_backward_workspace(g, H, F, grad_own != NULL,
+ * grad_att != NULL) bytes: the chunk partials of grad_own and the per-CTA
+ * partials of grad_att are reserved only for the outputs requested.
+ */
+int gno_gatv2_logits_backward_workspace(const gno_csr* g, int64_t H, int64_t F,
+                                        int with_grad_own, int with_grad_att,
+                                        size_t* bytes);
+int gno_gatv2_logits_backward(const gno_csr* g, const void* own, const void* other,
+                              int64_t other_rows, const void* att,
+                              const void* grad_logits, int64_t H, int64_t F,
+                              double negative_slope, void* grad_own, float* grad_att,
+                              int dtype, void* ws, size_t ws_bytes,
+                              gno_stream_t stream);
+
+/*
  * Integer form (int32 / int64 values, exact int64 accumulation): torch_scatter.scatter on
  * integer tensors — PyG's TopKPooling / to_dense_batch count nodes per graph with
  * scatter_add(batch.new_ones(n), batch, dim=0) (graph_benchmark/models/ptg_models.py:165-172).

@@ -14,8 +14,15 @@ flush is needed.  Algorithmic bytes are computed from the shapes (see `bytes_*`)
 counts the logits twice (the statistics pass reads them through perm, the apply pass again in
 original order).  Also reports launches per call (gno_launch_count) and the output of the fused
 op against baseline (b) at the timed size.
+
+The GATv2 rows (gno_b200.gatv2_logits forward and backward, and a whole layer step: logits, softmax
+and aggregate, forward, then torch.autograd.grad w.r.t. x_l, x_r and att) compare against native
+torch only: PyG's `(leaky_relu(x_l[src] + x_r[dst]) * att).sum(-1)`.  They also report
+torch.cuda.max_memory_allocated over the call.  A native run that does not fit in device memory is
+recorded as "oom".
 """
 import argparse
+import gc
 import json
 import os
 import statistics
@@ -99,6 +106,17 @@ def bytes_aggregate(n_out, e, H, C, s):
 def bytes_edge_dot(n, e, H, C, s):
     # per edge: gathered x row + ids + dst + H outputs; grad_out rows once per row
     return e * (H * C * s + 12 + H * s) + n * H * C * s
+
+
+def bytes_gatv2_fwd(n, e, H, C, s):
+    # per edge: gathered x_l row + gidx, erow, eid + the edge's H logits; x_r rows once per row
+    return e * (H * C * s + 12 + H * s) + n * H * C * s
+
+
+def bytes_gatv2_bwd(n_src, n_dst, e, H, C, s):
+    # two passes (dst plan: grad_x_r and grad_att; src plan: grad_x_l), each per edge: gathered
+    # row + ids + the edge's H grad_logits; per row: own row read, gradient row written
+    return 2 * e * (H * C * s + 12 + H * s) + 2 * (n_src + n_dst) * H * C * s
 
 
 # ---- baselines ----
@@ -290,16 +308,141 @@ def run(key, iters):
            {"(a) composed": ma, "(b) native torch": mb}, normwise_err_vs_native_fp32=errs)
 
 
+def native_logits(x_l, x_r, att, src, dst):
+    return (torch.nn.functional.leaky_relu(x_l[src] + x_r[dst], 0.2) * att).sum(-1)
+
+
+def peak_gb(fn):
+    """(torch.cuda.max_memory_allocated over one call, memory allocated before it), in GB."""
+    torch.cuda.synchronize()
+    before = torch.cuda.memory_allocated()
+    torch.cuda.reset_peak_memory_stats()
+    fn()
+    torch.cuda.synchronize()
+    return round(torch.cuda.max_memory_allocated() / 1e9, 3), round(before / 1e9, 3)
+
+
+def native_or_oom(fn, *args):
+    """fn(*args), or "oom" when it does not fit in device memory."""
+    try:
+        return fn(*args)
+    except torch.cuda.OutOfMemoryError:
+        pass
+    gc.collect()  # outside the handler: the traceback's frames no longer hold the partial results
+    torch.cuda.empty_cache()
+    return "oom"
+
+
+def run_gatv2(key, iters):
+    name, H, C, dtype = SHAPES[key]
+    n, e = B.WORKLOADS[name][:2]
+    ex, off = B.WORKLOADS[name][4:6]
+    s = torch.finfo(dtype).bits // 8
+    src, dst = B.make_graph(n, n, e, ex, off, DEV, 42)
+    g = torch.Generator(device=DEV).manual_seed(11)
+    x_l = torch.randn((n, H, C), generator=g, device=DEV).to(dtype)
+    x_r = torch.randn((n, H, C), generator=g, device=DEV).to(dtype)
+    att = torch.randn((H, C), generator=g, device=DEV).to(dtype)
+    gl = torch.randn((e, H), generator=g, device=DEV).to(dtype)
+    gout = torch.randn((n, H, C), generator=g, device=DEV).to(dtype)
+    base = {"shape": key, "nodes": n, "edges": e, "heads": H, "channels": C, "dtype": str(dtype)[6:],
+            "l2": "working set far larger than L2, no flush"}
+
+    def report(op, ms, abytes, n_launch, native_ms, peak, native_peak, err):
+        gbs = abytes / (ms * 1e-3) / 1e9
+        emit(op=op, ms=round(ms, 4), algorithmic_GB=round(abytes / 1e9, 3), achieved_GBps=round(gbs, 1),
+             frac_of_copy_peak=round(gbs / COPY_PEAK, 4), copy_peak_GBps=COPY_PEAK, launches_per_call=n_launch,
+             native_ms=native_ms if native_ms == "oom" else round(native_ms, 4),
+             speedup_vs_native=None if native_ms == "oom" else round(native_ms / ms, 2),
+             max_memory_allocated_GB=peak[0], allocated_before_GB=peak[1],
+             native_max_memory_allocated_GB=native_peak if native_peak == "oom" else native_peak[0],
+             normwise_err_vs_native=err, **base)
+
+    def native_err(got, names, want_fn):
+        """Normwise error of `got` against native torch in fp32, or in the shape's dtype when the
+        fp32 run does not fit in device memory."""
+        for dt in dict.fromkeys((torch.float32, dtype)):
+            want = native_or_oom(want_fn, dt)
+            if want != "oom":
+                return {"vs": f"native {str(dt)[6:]}", **{k: rel_err(a, b) for k, a, b in zip(names, got, want)}}
+        return "native oom"
+
+    # ---- logits forward
+    fused_fwd = lambda: gno_b200.gatv2_logits(x_l, x_r, att, src, dst)  # noqa: E731
+    nat_fwd = lambda: native_logits(x_l, x_r, att, src, dst)  # noqa: E731
+    got = fused_fwd()
+    err = native_err((got,), ("logits",),
+                     lambda dt: (native_logits(x_l.to(dt), x_r.to(dt), att.to(dt), src, dst),))
+    del got
+    ms = timeit(fused_fwd, iters)
+    peak = peak_gb(fused_fwd)
+    nl = launches(fused_fwd)
+    mb = native_or_oom(timeit, nat_fwd, iters)
+    pb = native_or_oom(peak_gb, nat_fwd)
+    report("gatv2_logits forward", ms, bytes_gatv2_fwd(n, e, H, C, s), nl, mb, peak, pb, err)
+
+    # ---- logits backward (grad of x_l, x_r and att through autograd.grad)
+    xs = [t.detach().requires_grad_() for t in (x_l, x_r, att)]
+    lf = gno_b200.gatv2_logits(*xs, src, dst)
+    bwd = lambda: torch.autograd.grad(lf, xs, gl, retain_graph=True)  # noqa: E731
+    got = bwd()
+    err = native_err(got, ("grad_x_l", "grad_x_r", "grad_att"), lambda dt: torch.autograd.grad(
+        native_logits(*[t.to(dt) for t in xs], src, dst), xs, gl.to(dt)))
+    del got
+    ms = timeit(bwd, iters)
+    peak = peak_gb(bwd)
+    nl = launches(bwd)
+    del lf
+
+    def native_bwd_time():
+        lb = native_logits(*xs, src, dst)
+        nb = lambda: torch.autograd.grad(lb, xs, gl, retain_graph=True)  # noqa: E731
+        return timeit(nb, iters), peak_gb(nb)
+    r = native_or_oom(native_bwd_time)
+    mb, pb = ("oom", "oom") if r == "oom" else r
+    report("gatv2_logits backward (grad x_l, x_r, att)", ms, bytes_gatv2_bwd(n, n, e, H, C, s), nl, mb, peak, pb,
+           err)
+
+    # ---- a GATv2 layer step: logits -> softmax -> aggregate, forward + backward w.r.t. x_l, x_r, att
+    def fused_layer():
+        ts = [t.detach().requires_grad_() for t in (x_l, x_r, att)]
+        lg = gno_b200.gatv2_logits(*ts, src, dst)
+        o = gno_b200.attention_aggregate(ts[0], gno_b200.softmax(lg, dst, num_nodes=n), src, dst, n)
+        return (o,) + torch.autograd.grad(o, ts, gout)
+
+    def native_layer(dt=dtype):
+        ts = [t.detach().to(dt).requires_grad_() for t in (x_l, x_r, att)]
+        lg = native_logits(*ts, src, dst)
+        o = native_aggregate(ts[0], native_softmax(lg, dst, n), src, dst, n)
+        return (o,) + torch.autograd.grad(o, ts, gout.to(dt))
+
+    got = fused_layer()
+    err = native_err(got, ("out", "grad_x_l", "grad_x_r", "grad_att"), native_layer)
+    del got
+    ms = timeit(fused_layer, iters)
+    peak = peak_gb(fused_layer)
+    nl = launches(fused_layer)
+    mb = native_or_oom(timeit, native_layer, iters)
+    pb = native_or_oom(peak_gb, native_layer)
+    total = (bytes_gatv2_fwd(n, e, H, C, s) + bytes_gatv2_bwd(n, n, e, H, C, s) + bytes_softmax_fwd(n, e, H, s)
+             + bytes_softmax_bwd(n, e, H, s) + 2 * bytes_aggregate(n, e, H, C, s) + bytes_edge_dot(n, e, H, C, s))
+    report("GATv2 layer step (logits + softmax + aggregate, forward + backward)", ms, total, nl, mb, peak, pb, err)
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=",".join(SHAPES))
     ap.add_argument("--iters", type=int, default=5)
+    ap.add_argument("--ops", default="attention,gatv2", help="attention (softmax, aggregate), gatv2 (logits, layer)")
     args = ap.parse_args()
     emit(op="card", **card())
+    runners = {"attention": run, "gatv2": run_gatv2}
     for k in args.only.split(","):
-        gno_b200.clear_caches()
-        torch.cuda.empty_cache()
-        try:
-            run(k, args.iters)
-        except Exception as ex:  # keep going: partial tables are still useful
-            print(json.dumps({"shape": k, "error": repr(ex)[:500]}), flush=True)
+        for op in args.ops.split(","):
+            gno_b200.clear_caches()
+            gc.collect()
+            torch.cuda.empty_cache()
+            try:
+                runners[op](k, args.iters)
+            except Exception as ex:  # keep going: partial tables are still useful
+                print(json.dumps({"shape": k, "ops": op, "error": repr(ex)[:500]}), flush=True)
