@@ -295,6 +295,81 @@ int gno_gatv2_logits_backward(const gno_csr* g, const void* own, const void* oth
                               gno_stream_t stream);
 
 /*
+ * Several aggregators over one neighbourhood in one pass (PNAConv.aggregate of PyG: a list of
+ * aggregators concatenated, then copies scaled by degree scalers; Corso et al., "Principal
+ * Neighbourhood Aggregation").  Codes of the aggregators and scalers, in output order:
+ */
+typedef enum gno_aggregator {
+  GNO_AGG_SUM = 0,
+  GNO_AGG_MEAN = 1,
+  GNO_AGG_MIN = 2,
+  GNO_AGG_MAX = 3,
+  GNO_AGG_VAR = 4,
+  GNO_AGG_STD = 5
+} gno_aggregator;
+typedef enum gno_scaler {
+  GNO_SCALE_IDENTITY = 0,
+  GNO_SCALE_AMPLIFICATION = 1,  /* log(d + 1) / avg_log */
+  GNO_SCALE_ATTENUATION = 2,    /* avg_log / log(d + 1) */
+  GNO_SCALE_LINEAR = 3,         /* d / avg_lin */
+  GNO_SCALE_INVERSE_LINEAR = 4  /* avg_lin / d */
+} gno_scaler;
+
+/*
+ * Forward over the dst-sorted plan: message m_e = x[gidx[k], :] of sorted edge k (edge id
+ * eid[k]); x [x_rows, T*F] contiguous (T towers of F columns).  With d = max(row length, 1):
+ *   sum = Σ m, mean = sum / d, var = Σ m² / d − mean², std = sqrt(relu(var) + 1e-5),
+ *   min / max with torch_scatter's rule (lowest edge wins a tie, NaN never wins, empty -> 0),
+ *   out[i, t*S*A*F + (s*A + a)*F + f] = agg_a · scale_s(d)      (out [N, T*S*A*F])
+ * aggs [n_aggs] and scalers [n_scalers] are host arrays of the codes above (1..8 each,
+ * duplicates allowed).  Σm and Σm² accumulate in fp32; rows cut by a chunk boundary combine
+ * their chunk partials in chunk order in fp64; the scale is applied in fp32 and each output is
+ * rounded once.  For the backward, optionally: int32 winners arg_min / arg_max [N, T*F]
+ * (original edge ids, arg_fill where nothing won; need min or max among aggs) and fp32 mean /
+ * var [N, T*F] (var before relu; both or neither).  No atomics: bit-reproducible.
+ * ws >= gno_multi_aggregate_workspace(g, T, F, aggs, n_aggs) bytes.
+ */
+int gno_multi_aggregate_workspace(const gno_csr* g, int64_t T, int64_t F,
+                                  const int* aggs, int n_aggs, size_t* bytes);
+int gno_multi_aggregate(const gno_csr* g, const void* x, int64_t x_rows, int64_t T,
+                        int64_t F, const int* aggs, int n_aggs, const int* scalers,
+                        int n_scalers, double avg_lin, double avg_log, void* out,
+                        int32_t* arg_min, int32_t* arg_max, float* mean, float* var,
+                        int64_t arg_fill, int dtype, void* ws, size_t ws_bytes,
+                        gno_stream_t stream);
+
+/*
+ * Backward of gno_multi_aggregate w.r.t. the messages (message form: gidx = eid = the plan's
+ * perm, x [E, T*F] in original edge order).  grad_out [N, T*S*A*F] in `dtype`; the winners
+ * and mean / var saved by the forward (winners of each requested extreme, mean / var when var or
+ * std is requested).  Per row, c_a = Σ_s scale_s · grad_out block (s, a),
+ * cv = c_var + c_std · [var > 0] / (2 std), and every edge e of the row gets
+ *   grad_x[e] = c_sum + c_mean / d + 2 cv (m_e − mean) / d + [e = argmin] c_min + [e = argmax] c_max
+ * Each element of grad_x [x_rows, T*F] that a kept edge owns is written once (no atomics); edges
+ * the plan dropped are not written.
+ */
+int gno_multi_aggregate_backward(const gno_csr* g, const void* x, int64_t x_rows,
+                                 int64_t T, int64_t F, const int* aggs, int n_aggs,
+                                 const int* scalers, int n_scalers, double avg_lin,
+                                 double avg_log, const void* grad_out,
+                                 const int32_t* arg_min, const int32_t* arg_max,
+                                 const float* mean, const float* var, void* grad_x,
+                                 int dtype, gno_stream_t stream);
+
+/*
+ * Node-level coefficients of the same backward (gather form, where grad_x[j] sums over the
+ * edges with source j): fp32 pq [N + 1, 2*T*F] gets rows [P | Q] for rows 0..N-1 with
+ *   P = c_sum + c_mean / d − 2 cv · mean / d,  Q = 2 cv / d
+ * (row N is left to the caller), and c_min / c_max [N, T*F] fp32 are written when non-NULL.
+ */
+int gno_multi_aggregate_coeffs(const gno_csr* g, int64_t T, int64_t F, const int* aggs,
+                               int n_aggs, const int* scalers, int n_scalers,
+                               double avg_lin, double avg_log, const void* grad_out,
+                               const int32_t* arg_min, const int32_t* arg_max,
+                               const float* mean, const float* var, float* pq,
+                               float* c_min, float* c_max, int dtype, gno_stream_t stream);
+
+/*
  * Integer form (int32 / int64 values, exact int64 accumulation): torch_scatter.scatter on
  * integer tensors — PyG's TopKPooling / to_dense_batch count nodes per graph with
  * scatter_add(batch.new_ones(n), batch, dim=0) (graph_benchmark/models/ptg_models.py:165-172).

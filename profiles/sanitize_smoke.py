@@ -45,5 +45,19 @@ k = torch.randint(0, 1 << 62, (70001,), device=dev, generator=g)
 gno_b200.sort_pairs(k, torch.arange(70001, device=dev, dtype=torch.int32), 0, 64)
 gno_b200.sort_pairs(k.to(torch.int32), None, 0, 32)
 gno_b200.segment_csr(torch.randn(1000, 6, device=dev, generator=g), torch.tensor([0, 0, 10, 500, 1000], device=dev), None, "max", True)
+# multi_aggregate: odd widths and towers, hub rows over several chunks, empty rows, dropped
+# destinations; forward and both backward forms
+avg = {"lin": 3.0, "log": 1.2}
+for dtype in (torch.float32, torch.bfloat16, torch.float16):
+    for (E, N, T, F) in ((3001, 40, 1, 7), (999, 300, 3, 5), (4097, 9, 2, 1), (2000, 64, 1, 100)):
+        dst = (torch.rand(E, device=dev, generator=g) ** 3 * N).long()
+        dst[::97] = N + 1
+        src = torch.randint(0, 333, (E,), device=dev, generator=g)
+        for form_src, rows in ((None, E), (src, 333)):
+            x = torch.randn(rows, T, F, device=dev, generator=g).to(dtype).requires_grad_(True)
+            out = gno_b200.multi_aggregate(x, dst, N, ("sum", "mean", "min", "max", "var", "std"),
+                                           ("identity", "amplification", "attenuation", "linear", "inverse_linear"),
+                                           avg, src=form_src)
+            torch.autograd.grad(out.sum(), x)
 torch.cuda.synchronize()
 print("sanitize smoke ok")
