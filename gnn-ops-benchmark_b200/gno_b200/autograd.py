@@ -13,6 +13,40 @@ segment-reduce kernel on a plan sorted by the SOURCE ids (cached like the forwar
 import torch
 
 from . import ops
+from .plan import plan_cache
+
+
+def _div_count(g, cnt, dim, dtype=None):
+    """g / max(cnt, 1), a 1-D cnt broadcast along dim: in fp32 from the exact integer count, rounded
+    once to `dtype` (default g's).  A 16-bit count is already wrong above 256 in bf16 and 2048 in
+    fp16, and inf above 65504."""
+    if cnt.dim() == 1:
+        shape = [1] * g.dim()
+        shape[dim] = -1
+        cnt = cnt.view(shape)
+    return (g.to(torch.float32) / cnt.clamp(min=1).to(torch.float32)).to(dtype or g.dtype)
+
+
+def _row_counts(index, n):
+    """Entries of a 1-D index per row in [0, n) (int64; out-of-range entries, which the forward
+    drops, are not counted): the cached forward plan's rowptr, so no extra pass."""
+    if index.numel() > ops._MAX_PLAN_EDGES:
+        return torch.bincount(index[(index >= 0) & (index < n)], minlength=n)
+    rowptr = plan_cache.get(index, n).rowptr
+    return rowptr[1:] - rowptr[:-1]
+
+
+def _in_range(index, n):
+    """(index, keep): keep is None when every entry lies in [0, n); otherwise the entries the forward
+    dropped are replaced by 0 (n > 0) and keep marks the others.  The range is memoised per index
+    tensor, so the common case costs one host read per index."""
+    if index.numel() == 0:
+        return index, None
+    lo, hi = ops._memo("idx_range", index, (), lambda: (int(index.min()), int(index.max())))
+    if lo >= 0 and hi < n:
+        return index, None
+    keep = (index >= 0) & (index < n)
+    return torch.where(keep, index, torch.zeros_like(index)), keep
 
 
 def _gather_dim(t, dim, index, like):
@@ -54,30 +88,41 @@ class _Scatter(torch.autograd.Function):
             shape[dim] += 1  # sentinel row for empty outputs, trimmed below
             g = grad_out.new_zeros(shape).scatter_(dim, arg, grad_out)
             return g.narrow(dim, 0, shape[dim] - 1), None, None, None, None
-        if reduce == "mul":
-            index, src, out = ctx.saved_tensors
-            g = _gather_dim(grad_out * out, dim, index, src) / src
-            return g.masked_fill_(g.isnan(), 0), None, None, None, None
-        (index,) = ctx.saved_tensors
+        saved = ctx.saved_tensors
+        index, n = saved[0], grad_out.size(dim)
+        if grad_out.numel() == 0 or index.numel() == 0:
+            # no output rows (every entry dropped) or no entries: nothing reaches src
+            return grad_out.new_zeros(ctx.shape), None, None, None, None
         like = grad_out.new_empty(ctx.shape)
         if reduce == "mean":
-            idx1 = index if index.dim() == 1 else None
-            if idx1 is not None:
-                cnt = torch.bincount(idx1, minlength=grad_out.size(dim)).clamp_(min=1).to(grad_out.dtype)
-                shape = [1] * grad_out.dim()
+            if index.dim() == 1:
+                cnt = _row_counts(index, n)
+            else:  # full-shape index: count in fp32 (exact to 2^24), not with 16-bit ones
+                ones = torch.ones(like.shape, dtype=torch.float32, device=like.device)
+                cnt = ops.scatter(ones, index, dim, None, n, "sum")
+            grad_out = _div_count(grad_out, cnt, dim)
+        elif reduce == "mul":
+            out = saved[2]
+            grad_out = grad_out.to(torch.float32) * out.to(torch.float32)
+        # entries the forward dropped get zero gradient; the native gathers never see them
+        index, keep = _in_range(index, n)
+        g = _gather_dim(grad_out, dim, index, like)
+        if reduce == "mul":
+            g = (g / saved[1].to(torch.float32)).to(like.dtype)
+            g.masked_fill_(g.isnan(), 0)
+        if keep is not None:
+            if keep.dim() == 1 and g.dim() > 1:
+                shape = [1] * g.dim()
                 shape[dim] = -1
-                grad_out = grad_out / cnt.view(shape)
-            else:
-                ones = torch.ones_like(like)
-                cnt = ops.scatter(ones, index, dim, None, grad_out.size(dim), "sum").clamp_(min=1)
-                grad_out = grad_out / cnt
-        return _gather_dim(grad_out, dim, index, like), None, None, None, None
+                keep = keep.view(shape)
+            g = g.masked_fill(~keep, 0)
+        return g, None, None, None, None
 
 
 class _GatherScatter(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, src_ids, dst_ids, dim_size, reduce):
-        ctx.reduce, ctx.n_src, ctx.dim_size = reduce, x.size(0), dim_size
+        ctx.reduce, ctx.n_src, ctx.dim_size, ctx.dtype = reduce, x.size(0), dim_size, x.dtype
         if reduce in ("min", "max"):
             out, arg = ops.gather_scatter(x, src_ids, dst_ids, dim_size, reduce, return_arg=True)
             ctx.save_for_backward(src_ids, arg)
@@ -91,6 +136,9 @@ class _GatherScatter(torch.autograd.Function):
     def backward(ctx, grad_out, *unused):
         reduce = ctx.reduce
         grad_out = grad_out.contiguous()
+        src_ids = ctx.saved_tensors[0]
+        if grad_out.numel() == 0 or src_ids.numel() == 0:
+            return grad_out.new_zeros((ctx.n_src,) + tuple(grad_out.shape[1:])), None, None, None, None
         if reduce in ("min", "max"):
             src_ids, arg = ctx.saved_tensors
             E = src_ids.numel()
@@ -99,13 +147,21 @@ class _GatherScatter(torch.autograd.Function):
             g = ops.scatter(grad_out, winner, 0, None, ctx.n_src, "sum")  # full-shape index, collisions
             return g, None, None, None, None
         src_ids, dst_ids = ctx.saved_tensors
+        plan = plan_cache.get(dst_ids, ctx.dim_size)      # the forward's plan
         if reduce == "mean":
-            cnt = torch.bincount(dst_ids, minlength=ctx.dim_size).clamp_(min=1).to(grad_out.dtype)
-            grad_out = grad_out / cnt.view(-1, 1)
+            # fp32 gradient into the transposed aggregation: divided and summed, rounded once
+            grad_out = _div_count(grad_out, plan.rowptr[1:] - plan.rowptr[:-1], 0, torch.float32)
         elif reduce != "sum":
             raise NotImplementedError("gather_scatter backward: sum/mean/min/max")
+        if plan.n_dropped:
+            # edges the forward dropped read a zero row appended to the gradient
+            n = ctx.dim_size
+            dst_ids = ops._memo("dst_in_range", dst_ids, (n,),
+                                lambda: torch.where((dst_ids >= 0) & (dst_ids < n), dst_ids, torch.full_like(dst_ids, n)))
+            grad_out = torch.cat([grad_out, grad_out.new_zeros((1,) + tuple(grad_out.shape[1:]))])
         # transposed aggregation: grad_x[s] = sum over edges with source s of grad_out[dst]
-        return ops.gather_scatter(grad_out, dst_ids, src_ids, ctx.n_src, "sum"), None, None, None, None
+        g = ops.gather_scatter(grad_out, dst_ids, src_ids, ctx.n_src, "sum")
+        return g.to(ctx.dtype), None, None, None, None
 
 
 class _SegmentCSR(torch.autograd.Function):
@@ -127,14 +183,15 @@ class _SegmentCSR(torch.autograd.Function):
     def backward(ctx, grad_out, *unused):
         grad_out = grad_out.contiguous()
         E = ctx.shape[0]
+        if grad_out.numel() == 0 or E == 0:
+            return grad_out.new_zeros(ctx.shape), None, None
         if ctx.reduce in ("min", "max"):
             (arg,) = ctx.saved_tensors
             g = grad_out.new_zeros([E + 1] + list(ctx.shape[1:])).scatter_(0, arg, grad_out)
             return g[:E], None, None
         (indptr,) = ctx.saved_tensors
         if ctx.reduce == "mean":
-            cnt = (indptr[1:] - indptr[:-1]).clamp(min=1).to(grad_out.dtype)
-            grad_out = grad_out / cnt.view([-1] + [1] * (grad_out.dim() - 1))
+            grad_out = _div_count(grad_out, indptr[1:] - indptr[:-1], 0)
         g = ops.gather_csr(grad_out, indptr)            # rows [0, indptr[-1]); zeros before indptr[0]
         if g.size(0) < E:                                # elements past the last pointer get no gradient
             g = torch.cat([g, g.new_zeros([E - g.size(0)] + list(g.shape[1:]))])
@@ -162,34 +219,45 @@ class _SpmmCSR(torch.autograd.Function):
     def backward(ctx, grad_out, *unused):
         grad_out = grad_out.contiguous()
         need_mat, need_val = ctx.needs_input_grad[3], ctx.needs_input_grad[2] and ctx.has_value
+        dtype = grad_out.dtype
         if ctx.reduce in ("min", "max"):
             col, arg, value, mat = ctx.saved_tensors
-            nnz = col.numel()
-            safe = arg.clamp(max=max(nnz - 1, 0))
+        else:
+            rowptr, col, value, mat = ctx.saved_tensors
+        nnz = col.numel()
+        if nnz == 0 or grad_out.numel() == 0:
+            return (None, None, torch.zeros_like(value) if need_val else None,
+                    torch.zeros_like(mat) if need_mat else None, None)
+        if ctx.reduce in ("min", "max"):
+            safe = arg.clamp(max=nnz - 1)
             hit = arg < nnz
             g_mat = g_val = None
+            # products and collisions in fp32, rounded once
+            g32 = grad_out.to(torch.float32)
             if need_mat:
-                w = grad_out if not ctx.has_value else grad_out * value[safe].to(grad_out.dtype)
+                w = g32 if not ctx.has_value else g32 * value[safe].to(torch.float32)
                 winner = torch.where(hit, col[safe], torch.full_like(arg, -1))
-                g_mat = ops.scatter(w.contiguous(), winner, 0, None, ctx.n_src, "sum")
+                g_mat = ops.scatter(w.contiguous(), winner, 0, None, ctx.n_src, "sum").to(dtype)
             if need_val:
-                contrib = torch.where(hit, grad_out * mat[col[safe], torch.arange(mat.size(1), device=mat.device)],
-                                      torch.zeros_like(grad_out))
-                g_val = torch.zeros(nnz + 1, dtype=grad_out.dtype, device=grad_out.device)
+                picked = mat[col[safe], torch.arange(mat.size(1), device=mat.device)].to(torch.float32)
+                contrib = torch.where(hit, g32 * picked, torch.zeros_like(g32))
+                g_val = torch.zeros(nnz + 1, dtype=torch.float32, device=grad_out.device)
                 g_val.index_add_(0, arg.reshape(-1).clamp(max=nnz), contrib.reshape(-1))
                 g_val = g_val[:nnz].to(value.dtype)
             return None, None, g_val, g_mat, None
-        rowptr, col, value, mat = ctx.saved_tensors
         if ctx.reduce == "mean":
-            cnt = (rowptr[1:] - rowptr[:-1]).clamp(min=1).to(grad_out.dtype)
-            grad_out = grad_out / cnt.view(-1, 1)
+            # fp32 gradient into the transposed product: divided and summed, rounded once
+            grad_out = _div_count(grad_out, rowptr[1:] - rowptr[:-1], 0, torch.float32)
         elif ctx.reduce not in ("sum", "add"):
             raise NotImplementedError("spmm backward: sum / mean / min / max")
-        g_mat = ops.spmm_csr_t(rowptr, col, value if ctx.has_value else None, grad_out, ctx.n_src) if need_mat else None
+        g_mat = None
+        if need_mat:
+            g_mat = ops.spmm_csr_t(rowptr, col, value if ctx.has_value else None, grad_out, ctx.n_src).to(dtype)
         g_val = None
         if need_val:
-            row = ops.csr_rows(rowptr, col.numel())
-            g_val = (grad_out.index_select(0, row) * mat.index_select(0, col)).sum(-1).to(value.dtype)
+            row = ops.csr_rows(rowptr, nnz)
+            g_val = (grad_out.index_select(0, row).to(torch.float32) *
+                     mat.index_select(0, col).to(torch.float32)).sum(-1).to(value.dtype)
         return None, None, g_val, g_mat, None
 
 

@@ -623,7 +623,7 @@ class DistAggregator:
         if reduce == "mean" and self.split in ("source", "hybrid"):
             if self._row_counts is None:
                 self._row_counts = torch.bincount(self.dst_local, minlength=self.n_out).clamp_(min=1)
-            out.div_(self._row_counts.to(out.dtype).view(-1, 1))
+            out.copy_(out.to(torch.float32) / self._row_counts.to(torch.float32).view(-1, 1))
         return (out, arg) if want_arg else out
 
     def aggregate(self, x_local, reduce="sum", return_arg=False, x_full=None, out=None, stage_bufs=None):
@@ -644,8 +644,8 @@ class DistAggregator:
                 ops.segment_reduce(p, buf, "sum", gidx=gidx, out=out, accumulate=c > 0)
             if reduce == "mean":
                 plan, _ = self.plan()
-                cnt = (plan.rowptr[1:] - plan.rowptr[:-1]).clamp_(min=1).to(out.dtype)
-                out.div_(cnt.view(-1, 1))
+                cnt = (plan.rowptr[1:] - plan.rowptr[:-1]).clamp_(min=1).to(torch.float32)
+                out.copy_(out.to(torch.float32) / cnt.view(-1, 1))
             return out
         plan, gidx = self.plan()
         if self.exchange_mode == "allgather_push":

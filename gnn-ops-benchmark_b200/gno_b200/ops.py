@@ -9,6 +9,7 @@ tensors are rejected (there is no fallback).
 """
 import collections
 import ctypes
+import math
 import os
 
 import torch
@@ -46,15 +47,17 @@ _memo_store = collections.OrderedDict()
 _pad_store = collections.OrderedDict()   # padded copies of x (_pad_for_gather): at most two
 
 
-def _memo(kind, t, extra, builder, capacity=32):
-    """Small LRU keyed on a tensor's identity/version (keeps the tensor alive)."""
+def _memo(kind, t, extra, builder, capacity=32, keep=None):
+    """Small LRU keyed on a tensor's identity/version (keeps the tensor alive).  `keep`: whatever
+    else the key names by address (a plan's rowptr), kept alive with the entry so that the address
+    cannot be handed to another tensor while the entry can still be hit."""
     key = (kind, t.data_ptr(), t._version, tuple(t.shape), t.stride(), t.dtype, t.device) + tuple(extra)
     hit = _memo_store.get(key)
     if hit is not None:
         _memo_store.move_to_end(key)
         return hit[0]
     val = builder()
-    _memo_store[key] = (val, t)
+    _memo_store[key] = (val, t, keep)
     while len(_memo_store) > capacity:
         _memo_store.popitem(last=False)
     return val
@@ -304,8 +307,9 @@ def scatter(src, index, dim=-1, out=None, dim_size=None, reduce="sum", return_ar
             if karg:
                 arg = (args[0] if B == 1 else torch.stack(args)).view(out_shape)
         if accumulate and red == GNO_MEAN:
-            cnt = (plan.rowptr[1:] - plan.rowptr[:-1]).clamp_(min=1).to(out.dtype)
-            out.div_(cnt.view([1] * dim + [N] + [1] * (len(out_shape) - dim - 1)))
+            # exact count, fp32 division, one rounding (a 16-bit count is wrong above 256 / 2048)
+            cnt = (plan.rowptr[1:] - plan.rowptr[:-1]).clamp_(min=1).to(torch.float32)
+            out.copy_(out.to(torch.float32) / cnt.view([1] * dim + [N] + [1] * (len(out_shape) - dim - 1)))
         if prev is not None:
             win = (arg != E) & ((out > prev) if red == GNO_MAX else (out < prev))
             prev.copy_(torch.where(win, out, prev))
@@ -387,7 +391,8 @@ def _scatter_chunked(src, idx1d, dim, out, N, reduce, red, want_arg, E):
         cnt = torch.bincount(idx1d[(idx1d >= 0) & (idx1d < N)], minlength=N)[:N].clamp_(min=1)
         shape = [1] * total.dim()
         shape[dim] = N
-        total = total / cnt.view(shape).to(total.dtype) if src.is_floating_point() else \
+        total = (total.to(torch.float32) / cnt.view(shape).to(torch.float32)).to(total.dtype) \
+            if src.is_floating_point() else \
             torch.div(total, cnt.view(shape), rounding_mode="floor")
     return total
 
@@ -621,7 +626,7 @@ def segment_csr(src, indptr, out=None, reduce="sum", return_arg=False):
     if indptr.dim() == 1:
         E = src.size(0)
         plan, lo, hi = _csr_plan(indptr, E)
-        x2 = src.contiguous().view(E, -1)[lo:hi]
+        x2 = src.contiguous().view(E, math.prod(src.shape[1:]))[lo:hi]   # -1 is ambiguous when E or F is 0
         r = segment_reduce(plan, x2, reduce, want_arg=want_arg, arg_fill=E)
         shape = [plan.N] + list(src.shape[1:])
         if want_arg:
@@ -672,7 +677,7 @@ def gather_csr(src, indptr):
         total = _memo("ptr_last", indptr, (), lambda: int(indptr[-1]))
         plan, lo, hi = _csr_plan(indptr, total)
         rows = _memo("erow64", plan.rowptr, (), lambda: plan.erow.to(torch.int64))
-        body = index_select(src.contiguous().view(M, -1), 0, rows)
+        body = index_select(src.contiguous().view(M, math.prod(src.shape[1:])), 0, rows)
         if lo:  # elements before the first pointer belong to no segment: zeros, as upstream's empty init
             body = torch.cat([body.new_zeros((lo, body.size(1))), body])
         return body.view([total] + list(src.shape[1:]))
@@ -753,7 +758,9 @@ def spmm(index, value, m, n, matrix, reduce="sum"):
                 check(lib.gno_permute_rows(_ptr(v), _ptr(plan.perm), _ptr(o), v.numel(),
                                            v.element_size(), _stream(v.device)))
             return o
-        w = _memo("perm_val", value, (plan.rowptr.data_ptr(), str(mat.dtype)), _permute)
+        # keyed on the plan's rowptr address: the entry keeps rowptr alive, so that a later plan
+        # cannot be given the same block and be served this plan's permutation
+        w = _memo("perm_val", value, (plan.rowptr.data_ptr(), str(mat.dtype)), _permute, keep=plan.rowptr)
     out = segment_reduce(plan, mat.contiguous(), reduce, gidx=gidx, weights=w)
     return out.squeeze(-1) if squeeze else out
 
@@ -805,7 +812,7 @@ def spmm_csr_t(rowptr, col, value, grad, n_cols):
                 check(lib.gno_permute_rows(_ptr(v), _ptr(plan.perm), _ptr(o), v.numel(),
                                            v.element_size(), _stream(v.device)))
             return o
-        w = _memo("perm_val", value, (plan.rowptr.data_ptr(), str(grad.dtype)), _permute)
+        w = _memo("perm_val", value, (plan.rowptr.data_ptr(), str(grad.dtype)), _permute, keep=plan.rowptr)
     return segment_reduce(plan, grad.contiguous(), "sum", gidx=gidx, weights=w)
 
 
