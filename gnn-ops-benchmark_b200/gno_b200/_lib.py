@@ -83,6 +83,15 @@ PROTOTYPES = {
     "gno_gatv2_logits_backward": (c_int, [POINTER(gno_csr), c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                           c_int64, c_int64, c_double, c_void_p, c_void_p, c_int, c_void_p,
                                           c_size_t, c_void_p]),
+    "gno_gatv2_attention_workspace": (c_int, [POINTER(gno_csr), c_int64, c_int64, POINTER(c_size_t)]),
+    "gno_gatv2_attention": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64,
+                                    c_double, c_double, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
+                                    c_void_p]),
+    "gno_gatv2_attention_backward_workspace": (c_int, [POINTER(gno_csr), c_int64, c_int64, c_int, c_int,
+                                                       POINTER(c_size_t)]),
+    "gno_gatv2_attention_backward": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
+                                             c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_double, c_void_p,
+                                             c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
     "gno_multi_aggregate_workspace": (c_int, [POINTER(gno_csr), c_int64, c_int64, c_void_p, c_int,
                                               POINTER(c_size_t)]),
     "gno_multi_aggregate": (c_int, [POINTER(gno_csr), c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int,

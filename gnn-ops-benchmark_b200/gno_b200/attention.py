@@ -6,9 +6,11 @@ gno_segment_softmax, gno_segment_reduce_heads, gno_edge_head_dot).
 A GATv2 layer computes per-edge, per-head logits [E, H] with `gatv2_logits`, normalises them over
 each destination's incoming edges with `softmax`, and aggregates
     out[i, h, :] = sum_{e: dst[e] = i} alpha[e, h] * x[src[e], h, :]
-with `attention_aggregate`, without materialising the [E, H, C] messages.  All three ops use the
-cached dst-sorted plan of the destination index; the backward passes that scatter to source nodes
-run on the cached src-sorted plan, so a training step builds two plans once and reuses them.
+with `attention_aggregate`, without materialising the [E, H, C] messages.  `gatv2_attention` is
+the same three steps in one pass (gno_gatv2_attention*): the logits and alpha are never stored.
+All these ops use the cached dst-sorted plan of the destination index; the backward passes that
+scatter to source nodes run on the cached src-sorted plan, so a training step builds two plans
+once and reuses them.
 """
 import collections
 import ctypes
@@ -273,14 +275,47 @@ class _GATv2Logits(torch.autograd.Function):
         return grad_l, grad_r, grad_att, None, None, None, None
 
 
-def _heads_view(t, name, H, C):
+def _heads_view(t, name, H, C, fn):
     """[N, H, C] or [N, H*C] -> [N, H*C] (checks H and C against att's)."""
     if t.dim() == 3:
         if t.size(1) != H or t.size(2) != C:
-            raise ValueError(f"gatv2_logits: {name} is [N, {t.size(1)}, {t.size(2)}], att [{H}, {C}]")
+            raise ValueError(f"{fn}: {name} is [N, {t.size(1)}, {t.size(2)}], att [{H}, {C}]")
     elif t.dim() != 2 or t.size(1) != H * C:
-        raise ValueError(f"gatv2_logits: {name} must be [N, {H}, {C}] or [N, {H * C}], got {tuple(t.shape)}")
+        raise ValueError(f"{fn}: {name} must be [N, {H}, {C}] or [N, {H * C}], got {tuple(t.shape)}")
     return t.reshape(t.size(0), H * C).contiguous()
+
+
+def _gatv2_args(fn, x_l, x_r, att, src, dst):
+    """The input conventions of gatv2_logits and gatv2_attention: checks, then (x_l [N_src, H*C],
+    x_r [N_dst, H*C], att [H*C] in x_l's dtype, src, dst, H, C)."""
+    ops._need_cuda(x_l, x_r, att, src, dst)
+    ops._dtype_id(x_l)
+    if x_r.dtype != x_l.dtype:
+        raise ValueError(f"{fn}: x_l is {x_l.dtype}, x_r {x_r.dtype}")
+    for name, t in (("src", src), ("dst", dst)):
+        if t.dtype != torch.int64 or t.dim() != 1:
+            raise ValueError(f"{fn}: {name} must be a 1-D int64 tensor")
+    E = src.numel()
+    if dst.numel() != E:
+        raise ValueError(f"{fn}: src and dst differ in length")
+    if att.dim() == 3 and att.size(0) == 1:
+        H, C = att.size(1), att.size(2)
+    elif att.dim() == 2:
+        H, C = att.shape
+    elif att.dim() == 1 and (x_l.dim() == 3 or x_r.dim() == 3):
+        H, C = (x_l if x_l.dim() == 3 else x_r).shape[1:]
+    elif att.dim() == 1:
+        raise ValueError(f"{fn}: a flat att needs x_l or x_r as [N, H, C] to know the heads")
+    else:
+        raise ValueError(f"{fn}: att must be [H, C], [1, H, C] or [H*C], got {tuple(att.shape)}")
+    if H == 0 or att.numel() != H * C:
+        raise ValueError(f"{fn}: att has {att.numel()} entries for {H} heads of {C}")
+    xl2 = _heads_view(x_l, "x_l", H, C, fn)
+    xr2 = _heads_view(x_r, "x_r", H, C, fn)
+    ops._check_range(src, xl2.size(0), f"{fn}: src")
+    ops._check_range(dst, xr2.size(0), f"{fn}: dst")
+    a2 = att.reshape(H * C).to(x_l.dtype).contiguous()
+    return xl2, xr2, a2, src.contiguous(), dst.contiguous(), H, C
 
 
 def gatv2_logits(x_l, x_r, att, src, dst, negative_slope=0.2):
@@ -294,31 +329,97 @@ def gatv2_logits(x_l, x_r, att, src, dst, negative_slope=0.2):
     x_l + x_r is formed in fp32 from the stored values; fp32 math, one rounding.  An out-of-range
     src or dst raises IndexError.  Differentiable w.r.t. x_l, x_r and att (x_l and x_r may be the
     same tensor); the backward recomputes the sums and saves no [E, ...] tensor."""
-    ops._need_cuda(x_l, x_r, att, src, dst)
-    ops._dtype_id(x_l)
-    if x_r.dtype != x_l.dtype:
-        raise ValueError(f"gatv2_logits: x_l is {x_l.dtype}, x_r {x_r.dtype}")
-    for name, t in (("src", src), ("dst", dst)):
-        if t.dtype != torch.int64 or t.dim() != 1:
-            raise ValueError(f"gatv2_logits: {name} must be a 1-D int64 tensor")
-    E = src.numel()
-    if dst.numel() != E:
-        raise ValueError("gatv2_logits: src and dst differ in length")
-    if att.dim() == 3 and att.size(0) == 1:
-        H, C = att.size(1), att.size(2)
-    elif att.dim() == 2:
-        H, C = att.shape
-    elif att.dim() == 1 and (x_l.dim() == 3 or x_r.dim() == 3):
-        H, C = (x_l if x_l.dim() == 3 else x_r).shape[1:]
-    elif att.dim() == 1:
-        raise ValueError("gatv2_logits: a flat att needs x_l or x_r as [N, H, C] to know the heads")
-    else:
-        raise ValueError(f"gatv2_logits: att must be [H, C], [1, H, C] or [H*C], got {tuple(att.shape)}")
-    if H == 0 or att.numel() != H * C:
-        raise ValueError(f"gatv2_logits: att has {att.numel()} entries for {H} heads of {C}")
-    xl2 = _heads_view(x_l, "x_l", H, C)
-    xr2 = _heads_view(x_r, "x_r", H, C)
-    ops._check_range(src, xl2.size(0), "gatv2_logits: src")
-    ops._check_range(dst, xr2.size(0), "gatv2_logits: dst")
-    a2 = att.reshape(H * C).to(x_l.dtype).contiguous()
-    return _GATv2Logits.apply(xl2, xr2, a2, src.contiguous(), dst.contiguous(), H, float(negative_slope))
+    xl2, xr2, a2, src, dst, H, _ = _gatv2_args("gatv2_logits", x_l, x_r, att, src, dst)
+    return _GATv2Logits.apply(xl2, xr2, a2, src, dst, H, float(negative_slope))
+
+
+class _GATv2Attention(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x_l, x_r, att, src, dst, H, slope):
+        N, F, dev = x_r.size(0), x_l.size(1), x_l.device
+        ctx.H, ctx.slope = H, slope
+        if src.numel() == 0 or F == 0:  # nothing to aggregate: zeros, and zero gradients below
+            out = torch.zeros((N, H, F // H), dtype=x_l.dtype, device=dev)
+            ctx.save_for_backward(x_l, x_r, att, src, dst, out, None, None)
+            return out
+        plan = plan_cache.get(dst, N)
+        csr = plan.csr(plan.sorted_ids(src), plan.perm)
+        out = torch.empty((N, H, F // H), dtype=x_l.dtype, device=dev)
+        m = torch.empty((N, H), dtype=torch.float32, device=dev)
+        s = torch.empty((N, H), dtype=torch.float32, device=dev)
+        nbytes = ctypes.c_size_t()
+        check(lib.gno_gatv2_attention_workspace(ctypes.byref(csr), H, F, ctypes.byref(nbytes)))
+        ws = _workspace(nbytes.value, dev)
+        with _on_device(dev):
+            check(lib.gno_gatv2_attention(ctypes.byref(csr), _ptr(x_l), x_l.size(0), _ptr(x_r), _ptr(att), H, F,
+                                          slope, EPS, _ptr(out), _ptr(m), _ptr(s), ops._dtype_id(x_l), _ptr(ws),
+                                          nbytes.value, _stream(dev)))
+        ctx.save_for_backward(x_l, x_r, att, src, dst, out, m, s)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        x_l, x_r, att, src, dst, out, m, s = ctx.saved_tensors
+        need_l, need_r, need_att = ctx.needs_input_grad[:3]
+        H, slope = ctx.H, ctx.slope
+        E, F, dev = src.numel(), x_l.size(1), x_l.device
+        if E == 0 or F == 0:
+            return (torch.zeros_like(x_l) if need_l else None, torch.zeros_like(x_r) if need_r else None,
+                    torch.zeros_like(att) if need_att else None, None, None, None, None)
+        g = grad_out.to(x_l.dtype).reshape(-1, F).contiguous()
+        grad_l = grad_r = grad_att = da = alpha = None
+        if need_r:
+            grad_r = torch.empty_like(x_r)
+        if need_att:
+            grad_att = torch.empty(F, dtype=torch.float32, device=dev)
+        if need_l:
+            da = torch.empty((E, H), dtype=x_l.dtype, device=dev)
+            alpha = torch.empty((E, H), dtype=x_l.dtype, device=dev)
+        # destination pass: grad_x_r, grad_att, and da / alpha for the source pass
+        plan = plan_cache.get(dst, x_r.size(0))
+        csr = plan.csr(plan.sorted_ids(src), plan.perm)
+        nbytes = ctypes.c_size_t()
+        check(lib.gno_gatv2_attention_backward_workspace(ctypes.byref(csr), H, F, need_r, need_att,
+                                                         ctypes.byref(nbytes)))
+        ws = _workspace(nbytes.value, dev)
+        with _on_device(dev):
+            check(lib.gno_gatv2_attention_backward(ctypes.byref(csr), _ptr(x_l), x_l.size(0), _ptr(x_r), _ptr(att),
+                                                   _ptr(out), _ptr(m), _ptr(s), _ptr(g), H, F, slope, _ptr(grad_r),
+                                                   _ptr(grad_att), _ptr(da), _ptr(alpha), ops._dtype_id(x_l),
+                                                   _ptr(ws), nbytes.value, _stream(dev)))
+        if need_l:
+            # source pass: the logit part through da, plus the transposed aggregation sum alpha * g[dst]
+            plan_t = plan_cache.get(src, x_l.size(0))
+            dst_t = plan_t.sorted_ids(dst)
+            grad_l = torch.empty_like(x_l)
+            _gatv2_backward(plan_t, dst_t, x_l, x_r, att, da, H, slope, grad_l, None)
+            grad_l += _aggregate(plan_t, dst_t, g, alpha, H, x_l.size(0))
+        if grad_att is not None:
+            grad_att = grad_att.to(att.dtype)
+        return grad_l, grad_r, grad_att, None, None, None, None
+
+
+def gatv2_attention(x_l, x_r, att, src, dst, negative_slope=0.2):
+    """A GATv2 layer's message passing in one op:
+        out[i, h, :] = sum_{e: dst[e] = i} alpha[e, h] * x_l[src[e], h, :]
+    with alpha = softmax over each destination (PyG 2.0.2: exp(a - max) / (sum exp + 1e-16), the
+    maximum by torch_scatter's rule as in `softmax`) of the logits
+        a[e, h] = sum_c att[h, c] * leaky_relu(x_l[src[e], h, c] + x_r[dst[e], h, c], negative_slope),
+    i.e. attention_aggregate(x_l, softmax(gatv2_logits(x_l, x_r, att, src, dst), dst,
+    num_nodes=N_dst), src, dst, N_dst), in one pass over the edges: each gathered x_l row serves
+    the logit and the weighted sum, and neither the [E, H] logits nor alpha are stored.  The
+    logits, the softmax statistics and the sum stay in fp32 and the output is rounded once, where
+    the three-op composition rounds the logits and alpha to a 16-bit dtype on the way.
+
+    Inputs as in `gatv2_logits`: x_l [N_src, H, C] or [N_src, H*C]; x_r [N_dst, H, C] or
+    [N_dst, H*C]; att [H, C], [1, H, C] or [H*C]; src / dst int64 [E]; fp32, fp16 or bf16.
+    Returns [N_dst, H, C] in x_l's dtype; destinations without an edge get 0.  An out-of-range
+    src or dst raises IndexError.  Differentiable w.r.t. x_l, x_r and att (x_l may be x_r); the
+    backward keeps no [E, ...] tensor from the forward, only out and fp32 [N_dst, H] statistics,
+    and builds the src-sorted plan only when x_l needs a gradient.
+
+    Not covered: attention dropout, return_attention_weights and edge features (GATv2Conv's
+    edge_dim).  Callers that need them use the three ops above, whose alpha is an explicit
+    tensor."""
+    xl2, xr2, a2, src, dst, H, C = _gatv2_args("gatv2_attention", x_l, x_r, att, src, dst)
+    return _GATv2Attention.apply(xl2, xr2, a2, src, dst, H, float(negative_slope))

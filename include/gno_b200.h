@@ -295,6 +295,56 @@ int gno_gatv2_logits_backward(const gno_csr* g, const void* own, const void* oth
                               gno_stream_t stream);
 
 /*
+ * A GATv2 layer's whole message passing in one pass over the dst-sorted plan of
+ * dst (gidx = src[perm], eid = perm): gno_gatv2_logits, gno_segment_softmax and
+ * gno_segment_reduce_heads fused, the way flash attention fuses score, softmax
+ * and weighted sum:
+ *   a[e, h]      = sum_c att[h*C + c] * leaky_relu(x_l[src, h*C + c] + x_r[dst, h*C + c])
+ *   alpha[e, h]  = exp(a - m[dst, h]) / s[dst, h]   (gno_segment_softmax's max rule)
+ *   out[i, h*C + c] = sum over the row's edges of alpha[e, h] * x_l[src, h*C + c]
+ * Each gathered x_l vector is loaded once and serves the logit and the weighted
+ * sum (online max / sum-of-exp rescaling).  Neither a nor alpha is written:
+ * out [N, F] in `dtype` (empty rows get 0) and the fp32 row statistics m [N, H]
+ * (the max after the empty-value rule) and s [N, H] (sum of exp(a - m) + eps)
+ * are, for the backward.  x_l [xl_rows, F], x_r [N, F], att [F] contiguous,
+ * F = H*C; a head may span at most 128 vectors of the widest load that divides
+ * it.  fp32 math, one rounding per output; atomic-free, bit-reproducible.
+ * E = 0 touches nothing.  ws >= gno_gatv2_attention_workspace(g, H, F) bytes.
+ */
+int gno_gatv2_attention_workspace(const gno_csr* g, int64_t H, int64_t F, size_t* bytes);
+int gno_gatv2_attention(const gno_csr* g, const void* x_l, int64_t xl_rows,
+                        const void* x_r, const void* att, int64_t H, int64_t F,
+                        double negative_slope, double eps, void* out, float* m,
+                        float* s, int dtype, void* ws, size_t ws_bytes,
+                        gno_stream_t stream);
+
+/*
+ * The destination pass of gno_gatv2_attention's backward, on the same plan.
+ * With D[i, h] = sum_c grad_out[i, h*C + c] * out[i, h*C + c], it recomputes a
+ * and alpha from m and s and forms
+ *   da[e, h]       = alpha * (sum_c grad_out[dst, h*C + c] * x_l[src, h*C + c] - D[dst, h])
+ *   grad_x_r[i, f] = att[f] * sum over the row's edges of da * leaky_relu'(z)   (empty rows 0)
+ *   grad_att[f]    = sum_e da * leaky_relu(z)                                  (fp32)
+ * and writes grad_logits = da and alpha [E, H] in original edge order, the
+ * inputs of the source pass: gno_gatv2_logits_backward (own = x_l, other = x_r,
+ * grad_logits = da) on the src plan gives the logit part of grad_x_l, and
+ * gno_segment_reduce_heads (x = grad_out, alpha) the rest.  grad_x_r, grad_att
+ * and the pair (grad_logits, alpha) may each be NULL, not all three.  No
+ * atomics: bit-reproducible.  ws >= gno_gatv2_attention_backward_workspace(g,
+ * H, F, grad_x_r != NULL, grad_att != NULL) bytes.
+ */
+int gno_gatv2_attention_backward_workspace(const gno_csr* g, int64_t H, int64_t F,
+                                           int with_grad_x_r, int with_grad_att,
+                                           size_t* bytes);
+int gno_gatv2_attention_backward(const gno_csr* g, const void* x_l, int64_t xl_rows,
+                                 const void* x_r, const void* att, const void* out,
+                                 const float* m, const float* s, const void* grad_out,
+                                 int64_t H, int64_t F, double negative_slope,
+                                 void* grad_x_r, float* grad_att, void* grad_logits,
+                                 void* alpha, int dtype, void* ws, size_t ws_bytes,
+                                 gno_stream_t stream);
+
+/*
  * Several aggregators over one neighbourhood in one pass (PNAConv.aggregate of PyG: a list of
  * aggregators concatenated, then copies scaled by degree scalers; Corso et al., "Principal
  * Neighbourhood Aggregation").  Codes of the aggregators and scalers, in output order:

@@ -20,6 +20,12 @@ and aggregate, forward, then torch.autograd.grad w.r.t. x_l, x_r and att) compar
 torch only: PyG's `(leaky_relu(x_l[src] + x_r[dst]) * att).sum(-1)`.  They also report
 torch.cuda.max_memory_allocated over the call.  A native run that does not fit in device memory is
 recorded as "oom".
+
+The fused rows (--ops fused) time gno_b200.gatv2_attention, the whole message passing in one op:
+its forward, its backward through torch.autograd.grad w.r.t. x_l, x_r and att, and a layer step
+(forward + backward), each against the three-op composition gatv2_logits -> softmax ->
+attention_aggregate in the same run, with launches, algorithmic bytes over the copy peak,
+max_memory_allocated and the normwise error of both against native torch in fp32.
 """
 import argparse
 import gc
@@ -429,14 +435,110 @@ def run_gatv2(key, iters):
     report("GATv2 layer step (logits + softmax + aggregate, forward + backward)", ms, total, nl, mb, peak, pb, err)
 
 
+def bytes_fused_fwd(n, e, H, C, s):
+    # per edge: gathered x_l row + erow, gidx; per row: x_r read, out written, fp32 (m, s) written
+    return e * (H * C * s + 8) + n * (2 * H * C * s + 8 * H)
+
+
+def bytes_fused_bwd(n_src, n_dst, e, H, C, s):
+    # dst pass: per edge x_l row + erow, gidx, eid + da, alpha written; per row x_r, g, out read,
+    # grad_x_r written, (m, s) read.  src pass: gno_gatv2_logits_backward (grad of x_l through da),
+    # the transposed aggregation alpha * g[dst], and their sum.
+    dst_pass = e * (H * C * s + 12 + 2 * H * s) + n_dst * (4 * H * C * s + 8 * H)
+    src_pass = e * (H * C * s + 12 + H * s) + 2 * n_src * H * C * s + bytes_aggregate(n_src, e, H, C, s)
+    return dst_pass + src_pass + 3 * n_src * H * C * s
+
+
+def run_fused(key, iters):
+    name, H, C, dtype = SHAPES[key]
+    n, e = B.WORKLOADS[name][:2]
+    ex, off = B.WORKLOADS[name][4:6]
+    s = torch.finfo(dtype).bits // 8
+    src, dst = B.make_graph(n, n, e, ex, off, DEV, 42)
+    g = torch.Generator(device=DEV).manual_seed(11)
+    x_l = torch.randn((n, H, C), generator=g, device=DEV).to(dtype)
+    x_r = torch.randn((n, H, C), generator=g, device=DEV).to(dtype)
+    att = torch.randn((H, C), generator=g, device=DEV).to(dtype)
+    gout = torch.randn((n, H, C), generator=g, device=DEV).to(dtype)
+    base = {"shape": key, "nodes": n, "edges": e, "heads": H, "channels": C, "dtype": str(dtype)[6:],
+            "l2": "working set far larger than L2, no flush"}
+
+    def composed(xl, xr, a):
+        lg = gno_b200.gatv2_logits(xl, xr, a, src, dst)
+        return gno_b200.attention_aggregate(xl, gno_b200.softmax(lg, dst, num_nodes=n), src, dst, n)
+
+    def fused(xl, xr, a):
+        return gno_b200.gatv2_attention(xl, xr, a, src, dst)
+
+    def native_fp32(with_grad):
+        ts = [t.detach().float().requires_grad_(with_grad) for t in (x_l, x_r, att)]
+        o = native_aggregate(ts[0], native_softmax(native_logits(*ts, src, dst), dst, n), src, dst, n)
+        return (o.detach(),) + (torch.autograd.grad(o, ts, gout.float()) if with_grad else ())
+
+    def errors(results, names, with_grad):
+        want = native_or_oom(native_fp32, with_grad)
+        if want == "oom":
+            return "native fp32 oom"
+        return {which: {k: rel_err(a, b) for k, a, b in zip(names, got, want)} for which, got in results.items()}
+
+    def report(op, ms, ms_comp, abytes, nl, nl_comp, peak, peak_comp, err):
+        gbs = abytes / (ms * 1e-3) / 1e9
+        emit(op=op, ms=round(ms, 4), composition_ms=round(ms_comp, 4), speedup_vs_composition=round(ms_comp / ms, 2),
+             algorithmic_GB=round(abytes / 1e9, 3), achieved_GBps=round(gbs, 1),
+             frac_of_copy_peak=round(gbs / COPY_PEAK, 4), copy_peak_GBps=COPY_PEAK, launches_per_call=nl,
+             composition_launches_per_call=nl_comp, max_memory_allocated_GB=peak[0], allocated_before_GB=peak[1],
+             composition_max_memory_allocated_GB=peak_comp[0], normwise_err_vs_native_fp32=err, **base)
+
+    # ---- forward
+    runs = {}
+    for which, fn in (("fused", fused), ("composition", composed)):
+        f = lambda fn=fn: fn(x_l, x_r, att)  # noqa: E731
+        runs[which] = (timeit(f, iters), launches(f), peak_gb(f), (f(),))
+    err = errors({k: v[3] for k, v in runs.items()}, ("out",), False)
+    (ms, nl, pk, _), (mc, nc, pc, _) = runs["fused"], runs["composition"]
+    runs.clear()
+    report("gatv2_attention forward", ms, mc, bytes_fused_fwd(n, e, H, C, s), nl, nc, pk, pc, err)
+
+    # ---- backward (grad x_l, x_r, att through autograd.grad)
+    names = ("grad_x_l", "grad_x_r", "grad_att")
+    for which, fn in (("fused", fused), ("composition", composed)):
+        xs = [t.detach().requires_grad_() for t in (x_l, x_r, att)]
+        o = fn(*xs)
+        bwd = lambda o=o, xs=xs: torch.autograd.grad(o, xs, gout, retain_graph=True)  # noqa: E731
+        runs[which] = (timeit(bwd, iters), launches(bwd), peak_gb(bwd), bwd())
+        del o, xs, bwd
+    want = native_or_oom(native_fp32, True)
+    err = "native fp32 oom" if want == "oom" else {
+        k: {nm: rel_err(a, b) for nm, a, b in zip(names, v[3], want[1:])} for k, v in runs.items()}
+    del want
+    (ms, nl, pk, _), (mc, nc, pc, _) = runs["fused"], runs["composition"]
+    runs.clear()
+    report("gatv2_attention backward (grad x_l, x_r, att)", ms, mc, bytes_fused_bwd(n, n, e, H, C, s), nl, nc,
+           pk, pc, err)
+
+    # ---- a GATv2 layer step on the fused op against the composition: forward + backward
+    for which, fn in (("fused", fused), ("composition", composed)):
+        def step(fn=fn):
+            ts = [t.detach().requires_grad_() for t in (x_l, x_r, att)]
+            o = fn(*ts)
+            return (o,) + torch.autograd.grad(o, ts, gout)
+        runs[which] = (timeit(step, iters), launches(step), peak_gb(step), step())
+    err = errors({k: v[3] for k, v in runs.items()}, ("out",) + names, True)
+    (ms, nl, pk, _), (mc, nc, pc, _) = runs["fused"], runs["composition"]
+    runs.clear()
+    report("GATv2 layer step on gatv2_attention (forward + backward)", ms, mc,
+           bytes_fused_fwd(n, e, H, C, s) + bytes_fused_bwd(n, n, e, H, C, s), nl, nc, pk, pc, err)
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default=",".join(SHAPES))
     ap.add_argument("--iters", type=int, default=5)
-    ap.add_argument("--ops", default="attention,gatv2", help="attention (softmax, aggregate), gatv2 (logits, layer)")
+    ap.add_argument("--ops", default="attention,gatv2",
+                    help="attention (softmax, aggregate), gatv2 (logits, layer), fused (gatv2_attention)")
     args = ap.parse_args()
     emit(op="card", **card())
-    runners = {"attention": run, "gatv2": run_gatv2}
+    runners = {"attention": run, "gatv2": run_gatv2, "fused": run_fused}
     for k in args.only.split(","):
         for op in args.ops.split(","):
             gno_b200.clear_caches()

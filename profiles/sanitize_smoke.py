@@ -59,5 +59,17 @@ for dtype in (torch.float32, torch.bfloat16, torch.float16):
                                            ("identity", "amplification", "attenuation", "linear", "inverse_linear"),
                                            avg, src=form_src)
             torch.autograd.grad(out.sum(), x)
+# gatv2_attention: odd and wide heads, hub rows over several chunks, empty rows, N_src != N_dst;
+# forward and backward
+for dtype in (torch.float32, torch.bfloat16, torch.float16):
+    for (E, n_src, n_dst, H, C) in ((3001, 50, 40, 3, 7), (999, 300, 200, 8, 33), (4097, 20, 9, 1, 1),
+                                    (2000, 70, 64, 2, 130)):
+        dst = (torch.rand(E, device=dev, generator=g) ** 3 * n_dst).long()
+        dst[dst % 5 == 3] = 0
+        src = torch.randint(0, n_src, (E,), device=dev, generator=g)
+        ts = [torch.randn(r, H, C, device=dev, generator=g).to(dtype).requires_grad_(True)
+              for r in (n_src, n_dst, 1)]
+        out = gno_b200.gatv2_attention(ts[0], ts[1], ts[2], src, dst)
+        torch.autograd.grad(out.sum(), ts)
 torch.cuda.synchronize()
 print("sanitize smoke ok")
